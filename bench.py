@@ -3,6 +3,13 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path
     python bench.py --impl reference [...]                         the reference's CPU path, bounded sample
+    python bench.py [...] --dump-outputs DIR                       also write what the last timed step computed
+
+`--dump-outputs DIR`: after the K timed steps, DIR/<name>.npy holds what a caller of the timed path receives
+from the last of them: `water` (the whole water grid in the run's precision) or, above DUMP_CELLS cells,
+`water_sample` (the cells at sample_cells(rows, cols): a fixed, seeded, sorted set of flat row-major indices),
+and the block's reductions `max_diff`, `masked_sum`, `total_drain`, `wet_cells` (float64). The DEM is
+generated from a fixed seed, so two builds given the same arguments can be compared file by file.
 
 One STEP = one convergence block of the reference's solver loop
 (/root/reference/src/WDPMCL.c:1054-1268): zero-threshold + snapshot, 1000 iterations of the nine
@@ -52,6 +59,35 @@ BLOCK_ITERS = 1000
 THRES_MM = 0.005
 NODATA = -99999.0
 MODULES = {"add": 0, "subtract": 1, "drain": 2}
+DUMP_CELLS = 1 << 22  # sampled water cells of --dump-outputs: 32 MiB in fp64
+DUMP_SEED = 20261020
+
+
+def sample_cells(rows: int, cols: int) -> np.ndarray:
+    """Flat row-major indices of the water cells --dump-outputs writes: all of them up to DUMP_CELLS, else a
+    fixed sample drawn from DUMP_SEED (sorted, without repeats)."""
+    n = rows * cols
+    if n <= DUMP_CELLS:
+        return np.arange(n, dtype=np.int64)
+    return np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, DUMP_CELLS, dtype=np.int64))
+
+
+def sampled_rows(idx: np.ndarray, cols: int, row0: int, block: np.ndarray) -> np.ndarray:
+    """Values of the sampled cells `idx` (sorted flat indices of the whole grid) that lie in `block`, the grid's rows
+    row0 .. row0 + len(block) - 1 (a stripe's owned rows), in index order."""
+    lo, hi = np.searchsorted(idx, [row0 * cols, (row0 + block.shape[0]) * cols])
+    return block.ravel()[idx[lo:hi] - row0 * cols]
+
+
+def dump_outputs(out_dir: Path, rows: int, cols: int, water: np.ndarray, r) -> None:
+    """Write the water grid (or its sample) and the block reductions `r` of the last timed step."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    if rows * cols <= DUMP_CELLS:
+        np.save(out_dir / "water.npy", water.reshape(rows, cols))
+    else:
+        np.save(out_dir / "water_sample.npy", water)
+    for name in ("max_diff", "masked_sum", "total_drain", "wet_cells"):
+        np.save(out_dir / f"{name}.npy", np.array([getattr(r, name)], dtype=np.float64))
 
 
 def host_threads() -> int:
@@ -146,6 +182,11 @@ def physical_gpu_index(local_rank: int) -> int:
 # --------------------------------------------------------------------------- reference arm
 
 
+def warn_no_reference(what: str) -> None:
+    print(f"bench.py: WARNING: the reference-derived binaries under oracle/_ref are not built (no reference checkout at "
+          f"build time, see oracle/pyoracle.py reference_dir()): {what}", file=sys.stderr)
+
+
 def cpu_kernel():
     """(callable iterate(w, d, n_iters), kind, threads) - the reference kernels if built, else the port."""
     from oracle import pyoracle as po
@@ -170,6 +211,8 @@ def cpu_kernel():
                                           C.c_double(NODATA), C.c_int(self.R), C.c_int(self.Cc), C.c_int(n),
                                           self.td.ctypes.data_as(C.c_void_p), C.c_int(0), C.c_int(0))
         return Runner
+
+    warn_no_reference("the CPU baseline times this repository's C port of the kernels (kind 'port')")
 
     class Runner:  # noqa: F811
         kind = "port"
@@ -434,6 +477,14 @@ def run_ours(args):
         if rank + 1 < world:
             nb = nrows - (o0 - r0) - orows
             water_host[o0 - r0 + orows:] = torch.from_numpy(parts[rank + 1][1][:nb])
+    if args.dump_outputs:  # the owned rows hold the state after the last timed step; stripes send their sampled cells to rank 0
+        water = sampled_rows(sample_cells(size, size), size, o0, owned_host.numpy())
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, (o0, water))
+            water = np.concatenate([p[1] for p in sorted(parts, key=lambda p: p[0])])
+        if rank == 0:
+            dump_outputs(args.dump_outputs, size, size, water, last)
     e2e_steps = max(1, min(args.steps, args.e2e_steps))
     barrier()
     t0 = time.perf_counter()
@@ -492,6 +543,8 @@ def run_ours(args):
                                 "sample": f"{Dw.shape[0]-2}x{Dw.shape[1]-2} centre window of the same DEM in the state after warm-up "
                                           f"(wet fraction {wet:.3f}), {n_it} iterations in {dt:.1f} s"}
         from oracle import pyoracle as po
+        if args.serial_baseline and module == ADD and po.ref_binary() is None:
+            warn_no_reference("no cpu_baseline_serial (it runs the unmodified reference program)")
         if args.serial_baseline and module == ADD and po.ref_binary() is not None:
             import shutil
             import tempfile
@@ -547,7 +600,13 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=12.0)
     ap.add_argument("--sample-size", type=int, default=2048)
     ap.add_argument("--ref-iters-per-step", type=int, default=100)
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="write the water grid (a fixed sample above 4 Mi cells) and reductions of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the reference arm has no such output")
     if args.impl == "reference":
         args.sample_size = args.sample_size_ref
         run_reference_arm(args)

@@ -4,15 +4,16 @@
                (oracle/wdpm_oracle_impl.h), padded ROW-major grids.
 * `RefCL`    : oracle/_ref/librunoffcl_ref.so - the verbatim reference kernel file
                compiled as C (oracle/ref_shim), padded COLUMN-major grids exactly
-               as WDPMCL.c:1129-1134 flattens them. Present only when
-               `make -C oracle` ran in a container that has /root/reference (the
-               built binary travels to the GPU box; the sources do not).
+               as WDPMCL.c:1129-1134 flattens them. Present only when the oracle
+               was built with a checkout of the reference (CentreForHydrology/WDPM)
+               at reference_dir(); the repository does not carry its sources.
 * `ref_binary()`: path of oracle/_ref/WDPMCL_ref, the unmodified reference host
                linked against the minicl stand-in runtime.
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
 import subprocess
 from pathlib import Path
 
@@ -24,11 +25,22 @@ SCHED_OPENCL, SCHED_SERIAL = 0, 1
 MODULES = {"add": ADD, "subtract": SUBTRACT, "drain": DRAIN}
 
 
+def reference_dir() -> Path | None:
+    """The reference checkout: WDPM_REFERENCE if set, else a directory `reference` beside this repository.
+    None when it is absent or cannot be read (an unreadable location is no reference, not an error)."""
+    ref = Path(os.environ.get("WDPM_REFERENCE") or HERE.parent.parent / "reference")
+    try:
+        return ref if (ref / "src" / "runoff.cl").is_file() else None
+    except OSError:
+        return None
+
+
 def build(force: bool = False) -> None:
-    """Compile the oracle (and oracle/_ref when /root/reference exists)."""
+    """Compile the oracle (and oracle/_ref when the reference checkout, reference_dir(), is there)."""
     target = HERE / "_build" / "libwdpm_oracle.so"
-    if force or not target.exists() or Path("/root/reference/src/runoff.cl").exists():
-        subprocess.run(["make", "-C", str(HERE)], check=True, capture_output=True)
+    ref = reference_dir()
+    if force or not target.exists() or ref is not None:
+        subprocess.run(["make", "-C", str(HERE), f"REF={ref or ''}"], check=True, capture_output=True)
 
 
 def _sfx(dtype) -> tuple[str, type]:

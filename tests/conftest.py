@@ -28,7 +28,7 @@ def refcl():
     from oracle import pyoracle
     pyoracle.build()
     if not pyoracle.RefCL.available():
-        pytest.skip("oracle/_ref/librunoffcl_ref.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/librunoffcl_ref.so not built (needs the reference checkout at build time: ../reference or $WDPM_REFERENCE)")
     return pyoracle.RefCL()
 
 

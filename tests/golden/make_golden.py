@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Regenerate tests/golden/ from the UNMODIFIED reference (run in the build
-container, where /root/reference exists; the GPU box only reads the fixtures).
+"""Regenerate tests/golden/ from the UNMODIFIED reference (needs a checkout of
+CentreForHydrology/WDPM at pyoracle.reference_dir(); the tests only read the fixtures).
 
-What it runs (oracle/_ref/WDPMCL_ref = /root/reference/src/WDPMCL.c compiled as is
+What it runs (oracle/_ref/WDPMCL_ref = <reference>/src/WDPMCL.c compiled as is
 and linked to the minicl stand-in runtime that executes the verbatim runoff.cl):
 
   validate_WDPM.sh's sequence on dem/basin5.asc, once per backend
@@ -14,11 +14,15 @@ and linked to the minicl stand-in runtime that executes the verbatim runoff.cl):
   (oracle/_ref/librunoffcl_ref.so), per module and precision
   -> crop_vectors.npz
 
+  tests/test_oracle.py's live cases (edge shapes, NODATA holes, LIVE_ITERS iterations from
+  totaldrain LIVE_TD0) through the verbatim kernel file, per module and precision: inputs,
+  outputs and totaldrain -> live_vectors.npz   [--live-only: this file alone]
+
   BASELINE.json configs[0] (basin5 Add 300 mm, rof 1.0, tol 1 mm, thr 0.005 mm; 320 000
   iterations, ~6 min on 8 threads through the OpenCL branch; its output file is
   byte-identical to the serial backend's) -> ref_opencl_add300.asc.gz / .txt   [--cfg1]
 
-Usage: python tests/golden/make_golden.py [--reuse DIR] [--cfg1]
+Usage: [WDPM_REFERENCE=<checkout>] python tests/golden/make_golden.py [--reuse DIR] [--cfg1] [--live-only]
        (DIR/rt{0,1}/{add,drain,sub}.{asc,txt}, DIR/cfg1/add300.{asc,txt})
 """
 import argparse
@@ -34,10 +38,14 @@ import numpy as np
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT))
-REF = Path("/root/reference")
+sys.path.insert(0, str(HERE.parent))
 
 from oracle import pyoracle as po  # noqa: E402
 from wdpm_b200 import ascgrid  # noqa: E402
+
+REF = po.reference_dir()
+if REF is None:
+    raise SystemExit("no reference checkout: put it beside this repository as `reference` or set WDPM_REFERENCE (it must hold src/runoff.cl)")
 
 
 def gz(src: Path, dst: Path):
@@ -60,12 +68,31 @@ def run_sequence(outdir: Path, rt: int):
         (outdir / f"{name}.txt").write_text(res.stdout)
 
 
+def live_vectors():
+    """test_oracle_matches_verbatim_kernel_live's cases through the verbatim kernels -> live_vectors.npz."""
+    from test_oracle import LIVE_ITERS, LIVE_TD0, MODS, live_cases
+    oracle, ref = po.Oracle(), po.RefCL()
+    out = {}
+    for dt, dn in ((np.float64, "f64"), (np.float32, "f32")):
+        for k, (_, _, D, W, outlet) in enumerate(live_cases(oracle, dt)):
+            out[f"{dn}_{k}_dem"], out[f"{dn}_{k}_w0"], out[f"{dn}_{k}_outlet"] = D, W, np.array(outlet, dtype=np.int32)
+            for mn, mod in MODS:
+                w = W.copy()
+                td = ref.iterate(w, D, -99999.0, mod, LIVE_ITERS, outlet=outlet, totaldrain=LIVE_TD0)
+                out[f"{mn}_{dn}_{k}_w"], out[f"{mn}_{dn}_{k}_td"] = w, np.array(td, dtype=dt)
+    np.savez_compressed(HERE / "live_vectors.npz", **out)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reuse", type=Path)
     ap.add_argument("--cfg1", action="store_true")
+    ap.add_argument("--live-only", action="store_true")
     args = ap.parse_args()
     po.build()
+    live_vectors()
+    if args.live_only:
+        return
     gz(REF / "dem" / "basin5.asc", HERE / "basin5.asc.gz")
     work = args.reuse or Path(tempfile.mkdtemp())
     for rt, backend in ((0, "serial"), (1, "opencl")):

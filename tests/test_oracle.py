@@ -1,14 +1,13 @@
 """CPU: pin the oracle (oracle/wdpm_oracle_impl.h) against the reference.
 
 1. raw-precision vectors produced by the VERBATIM runoff.cl (tests/golden/crop_vectors.npz);
-2. the verbatim kernels live, when oracle/_ref was built in this container;
+2. the verbatim kernels live, when oracle/_ref was built (a reference checkout at pyoracle.reference_dir());
 3. the unmodified WDPMCL.c's output files for validate_WDPM.sh's Add -> Drain -> Subtract sequence
    on basin5, both backends, byte for byte, through the host logic of wdpm_b200/wdpmcl.py;
 4. the validation/ goldens (validate_WDPM.sh:48-70) via a restatement of the awk checks, and via the
-   reference's own awk scripts when /root/reference is present.
+   reference's own awk scripts when that checkout is there.
 """
 import subprocess
-from pathlib import Path
 
 import numpy as np
 import pytest
@@ -33,18 +32,43 @@ def test_oracle_matches_verbatim_kernel_vectors(oracle, dn, dt, mn, mod):
     assert dt(td) == g[f"td_{mn}_{dn}"]
 
 
+# edge shapes with NODATA holes, Drain's totaldrain starting non-zero: run live through the verbatim kernels when
+# oracle/_ref is built, and stored from such a run in tests/golden/live_vectors.npz (make_golden.py writes it)
+LIVE_SEED, LIVE_SHAPES, LIVE_ITERS, LIVE_TD0 = 11, ((1, 1), (2, 5), (31, 47), (64, 96), (97, 33)), 40, 0.5
+
+
+def live_cases(oracle, dt):
+    """(rows, cols, D, W, outlet) for each of LIVE_SHAPES, drawn from LIVE_SEED."""
+    rng = np.random.default_rng(LIVE_SEED)
+    for rows, cols in LIVE_SHAPES:
+        D, W = random_case(rng, rows, cols, dt)
+        yield rows, cols, D, W, oracle.find_outlet(D) or (1, 1)
+
+
 @pytest.mark.parametrize("dt", [np.float64, np.float32])
 @pytest.mark.parametrize("mn,mod", MODS)
 def test_oracle_matches_verbatim_kernel_live(oracle, refcl, dt, mn, mod):
-    rng = np.random.default_rng(11)
-    for rows, cols in ((1, 1), (2, 5), (31, 47), (64, 96), (97, 33)):
-        D, W = random_case(rng, rows, cols, dt)
-        outlet = oracle.find_outlet(D) or (1, 1)
+    for rows, cols, D, W, outlet in live_cases(oracle, dt):
         a, b = W.copy(), W.copy()
-        ta = oracle.iterate(a, D, -99999.0, mod, 40, outlet=outlet, totaldrain=0.5)
-        tb = refcl.iterate(b, D, -99999.0, mod, 40, outlet=outlet, totaldrain=0.5)
+        ta = oracle.iterate(a, D, -99999.0, mod, LIVE_ITERS, outlet=outlet, totaldrain=LIVE_TD0)
+        tb = refcl.iterate(b, D, -99999.0, mod, LIVE_ITERS, outlet=outlet, totaldrain=LIVE_TD0)
         assert np.array_equal(a, b), (rows, cols)
         assert ta == tb
+
+
+@pytest.mark.parametrize("dn,dt", [("f64", np.float64), ("f32", np.float32)])
+@pytest.mark.parametrize("mn,mod", MODS)
+def test_oracle_matches_verbatim_kernel_stored(oracle, dn, dt, mn, mod):
+    """The live test's cases, inputs and outputs as the verbatim kernels produced them (tests/golden/live_vectors.npz)."""
+    if not (GOLDEN / "live_vectors.npz").exists():
+        pytest.skip("tests/golden/live_vectors.npz not generated yet (make_golden.py --live-only, with the reference checkout)")
+    g = np.load(GOLDEN / "live_vectors.npz")
+    for k, (rows, cols) in enumerate(LIVE_SHAPES):
+        D, w = g[f"{dn}_{k}_dem"], g[f"{dn}_{k}_w0"].copy()
+        assert D.dtype == dt and D.shape == (rows + 2, cols + 2)
+        td = oracle.iterate(w, D, -99999.0, mod, LIVE_ITERS, outlet=tuple(int(x) for x in g[f"{dn}_{k}_outlet"]), totaldrain=LIVE_TD0)
+        assert np.array_equal(w, g[f"{mn}_{dn}_{k}_w"]), (rows, cols)
+        assert dt(td) == g[f"{mn}_{dn}_{k}_td"], (rows, cols)
 
 
 def test_serial_add_equals_opencl_add(oracle):
@@ -127,8 +151,9 @@ def test_validation_sequence_matches_reference_outputs(oracle, basin5, tmp_path,
         path, text = _asc_text(hdr, rep.water, tmp_path)
         assert text == golden_text(f"ref_{backend_name}_{name}.asc.gz"), name
         _check_goldens(name, text)
-        awk_dir = Path("/root/reference/validation")
-        if awk_dir.exists():
+        ref = po.reference_dir()
+        if ref is not None and (ref / "validation").is_dir():
+            awk_dir = ref / "validation"
             script = {"add10": "add_test.awk", "drain": "drain_test.awk", "sub10": "subtract_test.awk"}[name]
             extra = {"add10": ["-v", "add_depth=10", "-v", "specified_patch_depth=0.420810"],
                      "drain": ["-v", "specified_drain_vol=97577.54", "-v", "drain_row=333", "-v", "drain_col=468",
