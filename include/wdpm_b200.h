@@ -41,6 +41,18 @@ extern "C" {
 #define WDPM_SUBTRACT 1
 #define WDPM_DRAIN 2
 
+/* Update schedule: which of the reference's two backends (its "cpu" flag) the arithmetic follows.
+ * OPENCL (0, the default of a zeroed config): the kernels of src/runoff.cl.
+ * SERIAL (1): the serial branch of src/WDPMCL.c. Add is the same as OPENCL. Subtract relaxes with
+ *   runoffs, the Add step (:1934-1964), instead of runoffsubtract. Drain relaxes as runoffdrain does and
+ *   then, after every whole iteration, empties the outlet's 3x3 neighbourhood (drain(), :1859-1897):
+ *   the water of its cells with dem > nodata and w > 0 is summed in row-major order and added to
+ *   totaldrain, and all nine cells are set to 0. wdpm_subpass stays a bare sub-pass; every other call
+ *   that iterates includes the emptying. One outlet only (wdpm_set_outlets refuses a set), and a fused
+ *   variant with more than one iteration per launch refuses Drain. */
+#define WDPM_SCHEDULE_OPENCL 0
+#define WDPM_SCHEDULE_SERIAL 1
+
 /* precision of the device arithmetic and of the host arrays */
 #define WDPM_F32 0
 #define WDPM_F64 1 /* the reference's precision (src/runoff.cl:1) */
@@ -81,7 +93,8 @@ typedef struct wdpm_config {
     int32_t iters_per_launch; /* fused kernel: iterations carried per HBM round trip (0 = default) */
     int32_t fused_variant;    /* fused kernel tiling variant (0 = auto; see wdpm_fused_variant_info) */
     int32_t fused_chunk_rows; /* owned rows per CTA, rounded up to a multiple of 3 (0 = auto) */
-    int32_t reserved[5];
+    int32_t schedule;         /* WDPM_SCHEDULE_* */
+    int32_t reserved[4];
 } wdpm_config;
 
 /* What one convergence block reports (src/WDPMCL.c:1239-1268). */

@@ -413,6 +413,55 @@ __device__ __forceinline__ void record_contact(const DrainState<T>& ds, int buff
     ev->valid = 1;
 }
 
+// ---------------------------------------------------------------------------
+// Serial-schedule Drain (include/wdpm_b200.h, WDPM_SCHEDULE_SERIAL): after every whole iteration the
+// reference's drain() (src/WDPMCL.c:1859-1897) sums the water of the outlet's 3x3 cells that are valid
+// and wet, in row-major order from 0, adds the sum to totaldrain and zeroes all nine cells. One outlet.
+// The outlet cell itself is valid: on the device it wears the mark (relax.cuh, outlet_mark).
+// In an event buffer the sum travels as one event in slot kWipeSlot, after the nine sub-pass slots of
+// a one-iteration launch, so that fold_events adds it after that iteration's contacts:
+// (total + got) + 0 == total + got, because total + got is never -0.0 (got >= +0).
+// ---------------------------------------------------------------------------
+
+constexpr int kWipeSlot = 9;
+static_assert(kWipeSlot < kEventsPerBuffer, "the wipe event follows the nine sub-pass slots of one iteration");
+
+template <typename T>
+__device__ __forceinline__ T outlet_wipe_sum(const T* w, const T* d, size_t pitch) {
+    T got = T(0);
+    for (int a = -1; a <= 1; a++)
+        for (int b = -1; b <= 1; b++) {
+            const T e = d[a * (ptrdiff_t)pitch + b], v = w[a * (ptrdiff_t)pitch + b];
+            if ((is_valid_elevation(e) || is_outlet(e)) && v > T(0)) got = got + v;
+        }
+    return got;
+}
+
+// One thread. Zeroes the nine cells of w that this solver's memory holds (a row stripe: its owned rows and the
+// halo copies of its neighbours' rows, which arrived with the neighbours' export of the same iteration); the
+// solver that owns the outlet's row first takes the sum. `direct` adds it to the total at once (colour kernel),
+// otherwise it goes to event buffer `buffer`.
+template <typename T>
+__global__ void k_outlet_wipe(T* __restrict__ w, const T* __restrict__ d, Geom g, DrainState<T> ds, int buffer, int direct) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    const int orow = ds.outlet_rc[0], ocol = ds.outlet_rc[1];
+    if (orow >= 0 && orow < ds.P) {
+        const size_t c = dev_index(g, orow, ocol);
+        const T got = outlet_wipe_sum(w + c, d + c, (size_t)g.pitch);
+        if (direct) {
+            ds.totaldrain[0] = ds.totaldrain[0] + got;
+        } else {
+            DrainEvent<T>* ev = event_slot(ds.events, ds.n_outlets, buffer, 0, kWipeSlot);
+            ev->w_outlet = got;
+            ev->w_centre = T(0);
+            ev->valid = 1;
+        }
+    }
+    for (int i = orow - 1; i <= orow + 1; i++)
+        if (i >= -kPadTop && i < g.nrows_dev - kPadTop)
+            for (int j = ocol - 1; j <= ocol + 1; j++) w[dev_index(g, i, j)] = T(0);
+}
+
 // A Drain tile whose 3x3 holds outlets (rare): relax it in place and record the contacts. Out of line
 // so that its arrays live on the stack of this call only. `owner`: this CTA owns the centre, so it
 // reports the events (halo copies recompute the same contacts). `slot`: sub-pass slot in the buffer.
@@ -1279,6 +1328,7 @@ struct ResidentParams {
     int n_tx;       // CTAs per grid row
     int n_iters;
     int launch_slot;    // drain event buffer of the first iteration
+    int serial_wipe;    // Drain, serial schedule: empty the outlet's 3x3 after every iteration (k_outlet_wipe)
     DrainState<T> ds;
 };
 
@@ -1302,16 +1352,42 @@ k_resident(const ResidentParams<T> p) {
         const int i = k / SC, j = k - i * SC;
         sd[k] = p.dem[base + (size_t)i * pitch + j];
     }
+    // Serial-schedule Drain: the outlet's 3x3 is emptied after every iteration (k_outlet_wipe). Iteration k's
+    // emptying happens while iteration k+1 stages its window: every CTA zeroes the cells its copy holds, and the
+    // CTA that owns the outlet - its window holds the whole 3x3 (halo >= 3 on every side) - first takes the sum.
+    // That CTA, not block 0, also folds the contact events: in iteration k+1 it folds iteration k's contacts
+    // (recorded by any CTA before the grid barrier) and then adds the sum, so the total grows as contacts of k,
+    // emptying of k, contacts of k+1, and nobody else touches it. The last iteration's emptying works on global
+    // memory after the last grid barrier, where no CTA reads the water any more.
+    const bool wipe = MODULE == kDrain && p.serial_wipe;
+    const int orow = wipe ? p.ds.outlet_rc[0] : 0, ocol = wipe ? p.ds.outlet_rc[1] : 0;
+    const bool wipe_owner = wipe && orow >= r_own && orow < r_own + p.TR && ocol >= c_own && ocol < c_own + p.TC;
+    const bool folder = wipe ? wipe_owner : blockIdx.x == 0;
     int cur = p.cur, evbuf = p.launch_slot;
     for (int it = 0; it < p.n_iters; it++) {
         const T* __restrict__ win = p.w[cur];
         T* __restrict__ wout = p.w[cur ^ 1];
-        if (MODULE == kDrain && blockIdx.x == 0) fold_events(p.ds, prev_event_slot(evbuf), tid, NTHREADS);
+        if (MODULE == kDrain && folder && !wipe) fold_events(p.ds, prev_event_slot(evbuf), tid, NTHREADS);
         for (int k = tid; k < SR * SC; k += NTHREADS) {
             const int i = k / SC, j = k - i * SC;
             sw[k] = win[base + (size_t)i * pitch + j];
         }
         __syncthreads();
+        if (wipe) {
+            if (wipe_owner && tid == 0) {
+                fold_events(p.ds, prev_event_slot(evbuf), 0, 1);
+                if (it > 0) {  // the launch before ended with its own emptying
+                    const int a = (orow - r0) * SC + (ocol - c0);
+                    p.ds.totaldrain[0] = p.ds.totaldrain[0] + outlet_wipe_sum(sw + a, sd + a, (size_t)SC);
+                }
+            }
+            __syncthreads();
+            if (it > 0 && tid < 9) {
+                const int i = orow - 1 + tid / 3 - r0, j = ocol - 1 + tid % 3 - c0;
+                if (i >= 0 && i < SR && j >= 0 && j < SC) sw[i * SC + j] = T(0);
+            }
+            __syncthreads();
+        }
 #pragma unroll 1
         for (int sub = 0; sub < 9; sub++) {
             const int oi = sub / 3, oj = sub - 3 * oi;       // tile-start offsets = (reference oi, oj) - 1
@@ -1344,7 +1420,15 @@ k_resident(const ResidentParams<T> p) {
         cur ^= 1;
         evbuf = next_event_slot(evbuf);
     }
-    if (MODULE == kDrain && blockIdx.x == 0) fold_events(p.ds, prev_event_slot(evbuf), tid, NTHREADS);
+    if (MODULE == kDrain && folder && !wipe) fold_events(p.ds, prev_event_slot(evbuf), tid, NTHREADS);
+    if (wipe_owner && tid == 0 && p.n_iters > 0) {
+        fold_events(p.ds, prev_event_slot(evbuf), 0, 1);
+        T* w = p.w[cur];
+        const size_t c = dev_index(p.g, orow, ocol);
+        p.ds.totaldrain[0] = p.ds.totaldrain[0] + outlet_wipe_sum(w + c, p.dem + c, pitch);
+        for (int a = -1; a <= 1; a++)
+            for (int b = -1; b <= 1; b++) w[c + a * (ptrdiff_t)pitch + b] = T(0);
+    }
 }
 
 }  // namespace wdpm

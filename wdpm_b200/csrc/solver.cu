@@ -58,6 +58,7 @@ struct FusedVariant {
     size_t smem;
     FusedLaunchFn<T> launch[3];        // per module; nullptr = this variant does not implement the module
     FusedLaunchFn<T> launch_clean[3];  // used instead while wdpm_solver::water_clean holds (nullptr = none)
+    FusedLaunchFn<T> launch_ref_add;   // fp64 variants with the sign-gated Add step: Add in the reference form (nullptr = launch[kAdd] is)
     cudaError_t (*prepare)();
 };
 
@@ -75,6 +76,10 @@ cudaError_t prepare_fused() {
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_fused<T, kSubtract, CFG, NTHREADS, MINB, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return e;
+    if constexpr (sizeof(T) == 8 && (OPT & kOptAddFast)) {
+        e = cudaFuncSetAttribute(k_fused<T, kAdd, CFG, NTHREADS, MINB, OPT & ~kOptAddFast>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) return e;
+    }
     return cudaFuncSetAttribute(k_fused<T, kDrain, CFG, NTHREADS, MINB, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
 }
 
@@ -89,6 +94,8 @@ FusedVariant<T> make_variant() {
     v.launch[kSubtract] = launch_fused<T, kSubtract, CFG, NTHREADS, MINB, OPT>;
     v.launch[kDrain] = launch_fused<T, kDrain, CFG, NTHREADS, MINB, OPT>;
     v.launch_clean[kAdd] = v.launch_clean[kSubtract] = v.launch_clean[kDrain] = nullptr;
+    v.launch_ref_add = nullptr;
+    if constexpr (sizeof(T) == 8 && (OPT & kOptAddFast)) v.launch_ref_add = launch_fused<T, kAdd, CFG, NTHREADS, MINB, OPT & ~kOptAddFast>;
     v.prepare = prepare_fused<T, CFG, NTHREADS, MINB, OPT>;
     return v;
 }
@@ -108,6 +115,10 @@ cudaError_t prepare_wa() {
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_fused_wa<T, kAdd, CFG, OPT | kOptNoGuard, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return e;
+    if constexpr (sizeof(T) == 8 && (OPT & kOptAddFast)) {
+        e = cudaFuncSetAttribute(k_fused_wa<T, kAdd, CFG, OPT & ~kOptAddFast, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) return e;
+    }
     if constexpr (!(OPT & kOptStagger)) {
         e = cudaFuncSetAttribute(k_fused_wa<T, kDrain, CFG, OPT & ~kOptDrainFast, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return e;
@@ -127,6 +138,8 @@ FusedVariant<T> make_wa_variant() {
     v.launch[kSubtract] = launch_wa<T, kSubtract, CFG, OPT, MINB>;
     v.launch_clean[kAdd] = (OPT & kOptAddFast) ? launch_wa<T, kAdd, CFG, OPT | kOptNoGuard, MINB> : nullptr;
     v.launch_clean[kSubtract] = nullptr;
+    v.launch_ref_add = nullptr;
+    if constexpr (sizeof(T) == 8 && (OPT & kOptAddFast)) v.launch_ref_add = launch_wa<T, kAdd, CFG, OPT & ~kOptAddFast, MINB>;
     // Drain: the reference form of the step, and - fp64, while the water is known to hold no -0.0 (water_clean) - the
     // folded-gate form (relax.cuh, push_drain_fast). Not with the staggered schedule.
     if constexpr (OPT & kOptStagger) {
@@ -213,6 +226,11 @@ const std::vector<FusedVariant<float>>& fused_variants<float>() {
 struct wdpm_solver {
     wdpm_config cfg{};
     int dtype = WDPM_F64, module = WDPM_ADD;
+    int schedule = WDPM_SCHEDULE_OPENCL;
+    // the module whose relax arithmetic the kernels run: the serial schedule's Subtract relaxes with the Add step
+    // (runoffs, src/WDPMCL.c:1934-1964, is runoffadd bit for bit on every input the solver takes: relax.cuh,
+    // rewrite (1), and the host macro's tie rule differs from mini's only on signed zeros that cannot occur there)
+    int relax = WDPM_ADD;
     size_t esize = 8;
     Geom g{};
     int kernel = WDPM_KERNEL_COLOUR;
@@ -236,6 +254,12 @@ struct wdpm_solver {
     // True after a block prologue with a zero threshold > 0 (WDPMCL.c:1055-1065 wipes negatives and -0.0)
     // provided the last upload put no water on invalid cells (invalid_dry); the kernels preserve both.
     bool water_clean = false, invalid_dry = false;
+    // negzero_free: no valid cell holds -0.0. The fp64 sign-gated Add step (relax.cuh, push_add_fast) would turn a
+    // -0.0 neighbour at h == +0 into +0.0; the Add module never sees one (apply_add rewrites every valid cell), but
+    // the serial schedule's Subtract can (water uploaded without apply_subtract, zero threshold 0). While this is
+    // false such a solver runs a reference form of the Add step. True after apply_subtract and after a block
+    // prologue with a zero threshold > 0; no relax step creates a -0.0 (x - x = +0, +0 + -0 = +0).
+    bool negzero_free = false;
     int* d_dirty = nullptr;   // device flag of k_check_invalid_water
 
     // Drain outlets (kernels.cuh "Drain bookkeeping"): capacity kMaxOutlets
@@ -248,6 +272,7 @@ struct wdpm_solver {
     bool marks_applied = false;
     bool have_outlet = false;
     int launch_slot = 0;       // drain event buffer of the next launch (kernels.cuh, kEventSlots)
+    bool wipe_due = false;     // serial-schedule Drain: the last launched iteration's outlet emptying is still to come
 
     BlockPartial* partials = nullptr;
     BlockPartial* d_result = nullptr;
@@ -300,6 +325,25 @@ DrainState<T> drain_state(wdpm_solver* s) {
     return ds;
 }
 
+bool serial_drain(const wdpm_solver* s) { return s->schedule == WDPM_SCHEDULE_SERIAL && s->module == WDPM_DRAIN; }
+
+// Serial-schedule fp64 Subtract on water that may hold -0.0 (wdpm_solver::negzero_free): the Add step must keep
+// the reference's gate.
+bool needs_ref_add(const wdpm_solver* s) { return s->dtype == WDPM_F64 && s->relax == WDPM_ADD && s->module != WDPM_ADD && !s->negzero_free; }
+
+// Serial-schedule Drain: empty the outlet's 3x3 after the iteration that produced w[cur] (kernels.cuh,
+// k_outlet_wipe). `direct`: add the sum to the total at once (colour kernel); otherwise it goes into the event
+// buffer of that iteration's launch, after its contacts, and is folded with them.
+template <typename T>
+int outlet_wipe(wdpm_solver* s, bool direct) {
+    k_outlet_wipe<T><<<1, 32, 0, s->stream>>>(static_cast<T*>(s->w[s->cur]), static_cast<const T*>(s->dem), s->g, drain_state<T>(s),
+                                              prev_event_slot(s->launch_slot), direct ? 1 : 0);
+    s->launches++;
+    s->wipe_due = false;
+    CUDA_TRY(cudaGetLastError());
+    return WDPM_OK;
+}
+
 constexpr int kMaxOutlets = WDPM_MAX_OUTLETS;
 constexpr size_t kFlagsBytes = 256;  // HaloFlags, padded; the drain event buffers follow in the same allocation
 
@@ -320,7 +364,7 @@ int colour_subpass(wdpm_solver* s, int oi, int oj) {
     T* w = static_cast<T*>(s->w[s->cur]);
     const T* d = static_cast<const T*>(s->dem);
     DrainState<T> ds = drain_state<T>(s);
-    switch (s->module) {
+    switch (s->relax) {
         case WDPM_ADD: k_colour<T, kAdd><<<grid, block, 0, s->stream>>>(w, d, s->g, oi, oj, ds); break;
         case WDPM_SUBTRACT: k_colour<T, kSubtract><<<grid, block, 0, s->stream>>>(w, d, s->g, oi, oj, ds); break;
         default: k_colour<T, kDrain><<<grid, block, 0, s->stream>>>(w, d, s->g, oi, oj, ds); break;
@@ -332,12 +376,17 @@ int colour_subpass(wdpm_solver* s, int oi, int oj) {
 
 template <typename T>
 int colour_iterations(wdpm_solver* s, int n) {
-    for (int it = 0; it < n; it++)
+    for (int it = 0; it < n; it++) {
         for (int oi = 1; oi <= 3; oi++)
             for (int oj = 1; oj <= 3; oj++) {
                 const int rc = colour_subpass<T>(s, oi, oj);
                 if (rc) return rc;
             }
+        if (serial_drain(s)) {
+            const int rc = outlet_wipe<T>(s, true);
+            if (rc) return rc;
+        }
+    }
     return WDPM_OK;
 }
 
@@ -375,7 +424,8 @@ int fused_launch_only(wdpm_solver* s);
 
 template <typename T>
 FusedLaunchFn<T> pick_launch(const wdpm_solver* s, const FusedVariant<T>& v) {
-    return (s->water_clean && v.launch_clean[s->module]) ? v.launch_clean[s->module] : v.launch[s->module];
+    if (needs_ref_add(s) && v.launch_ref_add) return v.launch_ref_add;
+    return (s->water_clean && v.launch_clean[s->relax]) ? v.launch_clean[s->relax] : v.launch[s->relax];
 }
 
 template <typename T>
@@ -397,17 +447,29 @@ int fused_iterations(wdpm_solver* s, int n) {
             k_halo_wait<<<1, 32, 0, s->stream>>>(s->flags, s->above.present, s->below.present, s->epoch, s->halo_timeout_ns);
             s->launches++;
         }
+        // Serial-schedule Drain: the previous iteration's emptying. A row stripe does it after the wait above: its
+        // copy of a neighbour's rows of the 3x3 has then arrived (with values from before the emptying), and every
+        // stripe that holds one of the nine cells zeroes its own copy.
+        if (s->wipe_due) {
+            const int rc = outlet_wipe<T>(s, false);
+            if (rc) return rc;
+        }
         set_halo_export<T>(s, p);  // the launch also pushes the halo rows and raises the neighbours' flags
         CUDA_TRY(pick_launch<T>(s, v)(p, s->n_strips * s->n_chunks, s->stream));
         s->launches++;
         s->cur ^= 1;
         s->launch_slot = next_event_slot(s->launch_slot);
+        s->wipe_due = serial_drain(s);
     }
     if (s->module == WDPM_DRAIN && n_launch > 0) {
         if (s->stripe && (s->above.present || s->below.present)) {
             // the neighbours' last iteration records contacts with my outlets in my buffers: wait for it
             k_halo_wait<<<1, 32, 0, s->stream>>>(s->flags, s->above.present, s->below.present, s->epoch, s->halo_timeout_ns);
             s->launches++;
+        }
+        if (s->wipe_due) {
+            const int rc = outlet_wipe<T>(s, false);
+            if (rc) return rc;
         }
         k_fold_events<T><<<1, 256, 0, s->stream>>>(drain_state<T>(s), prev_event_slot(s->launch_slot));
         s->launches++;
@@ -437,6 +499,7 @@ int fused_launch_only(wdpm_solver* s) {
     s->launches++;
     s->cur ^= 1;
     s->launch_slot = next_event_slot(s->launch_slot);
+    s->wipe_due = serial_drain(s);
     return WDPM_OK;  // Drain: the contacts are folded by the next launch, or by phase 1 (fold_last_launch)
 }
 
@@ -445,6 +508,10 @@ int fused_launch_only(wdpm_solver* s) {
 template <typename T>
 int fold_last_launch(wdpm_solver* s) {
     if (s->module != WDPM_DRAIN) return WDPM_OK;
+    if (s->wipe_due) {  // serial schedule: every stripe's copy of the last iteration's rows is in place by now
+        const int rc = outlet_wipe<T>(s, false);
+        if (rc) return rc;
+    }
     k_fold_events<T><<<1, 256, 0, s->stream>>>(drain_state<T>(s), prev_event_slot(s->launch_slot));
     s->launches++;
     CUDA_TRY(cudaGetLastError());
@@ -466,6 +533,7 @@ cudaError_t launch_resident(wdpm_solver* s, int n) {
     p.n_tx = s->res_ntx;
     p.n_iters = n;
     p.launch_slot = s->launch_slot;
+    p.serial_wipe = serial_drain(s) ? 1 : 0;
     p.ds = drain_state<T>(s);
     void* args[] = {&p};
     auto kern = k_resident<T, MODULE, kResidentThreads>;  // shared-memory limit set in wdpm_create (resident_fits)
@@ -485,7 +553,7 @@ bool resident_fits(const wdpm_solver* s) {
 
 template <typename T>
 bool resident_fits_module(const wdpm_solver* s) {
-    switch (s->module) {
+    switch (s->relax) {
         case WDPM_ADD: return resident_fits<T, kAdd>(s);
         case WDPM_SUBTRACT: return resident_fits<T, kSubtract>(s);
         default: return resident_fits<T, kDrain>(s);
@@ -496,7 +564,7 @@ template <typename T>
 int resident_iterations(wdpm_solver* s, int n) {
     if (n <= 0) return WDPM_OK;
     cudaError_t e;
-    switch (s->module) {
+    switch (s->relax) {
         case WDPM_ADD: e = launch_resident<T, kAdd>(s, n); break;
         case WDPM_SUBTRACT: e = launch_resident<T, kSubtract>(s, n); break;
         default: e = launch_resident<T, kDrain>(s, n); break;
@@ -518,6 +586,8 @@ int resident_iterations(wdpm_solver* s, int n) {
 
 template <typename T>
 int iterate_t(wdpm_solver* s, int n) {
+    // the resident kernel's fp64 Add step is the sign-gated one: the colour kernel runs the reference form instead
+    if (s->kernel == WDPM_KERNEL_RESIDENT && needs_ref_add(s)) return colour_iterations<T>(s, n);
     if (s->kernel == WDPM_KERNEL_RESIDENT) return resident_iterations<T>(s, n);
     if (s->kernel == WDPM_KERNEL_FUSED) return fused_iterations<T>(s, n);
     return colour_iterations<T>(s, n);
@@ -540,6 +610,7 @@ int block_begin_t(wdpm_solver* s) {
         s->launches++;
     }
     if (s->cfg.zero_threshold > 0.0 && s->invalid_dry) s->water_clean = true;  // no negative water, no -0.0 left (see wdpm_solver)
+    if (s->cfg.zero_threshold > 0.0) s->negzero_free = true;
     CUDA_TRY(cudaMemsetAsync(s->d_dirty, 0, sizeof(int), s->stream));
     k_block_prologue<T><<<grid_for(n, 256, s->sm_count), 256, 0, s->stream>>>(
         static_cast<T*>(s->w[s->cur]), static_cast<T*>(s->oldw), static_cast<const T*>(s->dem), n, (T)s->cfg.zero_threshold, s->d_dirty);
@@ -663,6 +734,8 @@ int apply_outlet_marks(wdpm_solver* s, bool on) {
 // next block prologue; whether invalid cells are dry is established here (one pass, the callers synchronise anyway).
 int refresh_water_flags(wdpm_solver* s) {
     s->water_clean = false;
+    s->negzero_free = false;
+    s->wipe_due = false;  // new water: an emptying still pending belonged to the old one
     const long long n = s->g.cells_dev();
     const int grid = grid_for(n, 256, s->sm_count);
     CUDA_TRY(cudaMemsetAsync(s->d_dirty, 0, sizeof(int), s->stream));
@@ -725,6 +798,7 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
     if (cfg->dtype != WDPM_F32 && cfg->dtype != WDPM_F64) return fail(WDPM_E_ARG, "dtype must be WDPM_F32 or WDPM_F64");
     if (cfg->module < WDPM_ADD || cfg->module > WDPM_DRAIN) return fail(WDPM_E_ARG, "unknown module");
     if (cfg->kernel < WDPM_KERNEL_AUTO || cfg->kernel > WDPM_KERNEL_RESIDENT) return fail(WDPM_E_ARG, "unknown kernel selector");
+    if (cfg->schedule != WDPM_SCHEDULE_OPENCL && cfg->schedule != WDPM_SCHEDULE_SERIAL) return fail(WDPM_E_ARG, "unknown schedule");
     const bool is_stripe = cfg->stripe_rows > 0;
     if (is_stripe) {
         if (cfg->stripe_row0 < 0 || cfg->stripe_row0 % 3 != 0) return fail(WDPM_E_ARG, "stripe_row0 must be a non-negative multiple of 3");
@@ -751,6 +825,8 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
     s->cfg = *cfg;
     s->dtype = cfg->dtype;
     s->module = cfg->module;
+    s->schedule = cfg->schedule;
+    s->relax = (cfg->schedule == WDPM_SCHEDULE_SERIAL && cfg->module == WDPM_SUBTRACT) ? WDPM_ADD : cfg->module;
     s->esize = cfg->dtype == WDPM_F64 ? 8 : 4;
     s->device = cfg->device;
     cudaDeviceProp prop;
@@ -798,8 +874,8 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
         W = v.W; TWV = v.TWV; HL = v.HL; K = v.K; NT = v.NT; minb = v.minb; prepare = v.prepare;
     }
     {
-        const bool has_module = s->dtype == WDPM_F64 ? fused_variants<double>()[s->variant].launch[s->module] != nullptr
-                                                     : fused_variants<float>()[s->variant].launch[s->module] != nullptr;
+        const bool has_module = s->dtype == WDPM_F64 ? fused_variants<double>()[s->variant].launch[s->relax] != nullptr
+                                                     : fused_variants<float>()[s->variant].launch[s->relax] != nullptr;
         if (!has_module) { delete s; return fail(WDPM_E_UNSUPPORTED, "this fused variant does not implement the module (warp-autonomous variants: Add and Subtract)"); }
     }
     if (s->kernel == WDPM_KERNEL_FUSED) {
@@ -808,6 +884,8 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
     }
 
     if (is_stripe && K != 1) { delete s; return fail(WDPM_E_UNSUPPORTED, "stripes need a fused variant with one iteration per launch"); }
+    // the outlet's emptying sits between two iterations, and its event after the nine sub-pass slots of one iteration
+    if (serial_drain(s) && s->kernel == WDPM_KERNEL_FUSED && K != 1) { delete s; return fail(WDPM_E_UNSUPPORTED, "serial-schedule Drain needs a fused variant with one iteration per launch"); }
 
     // geometry (the tests' schedule emulator uses the same formulas). A stripe is a grid of P padded
     // rows whose halo rows live in the row margins above and below.
@@ -1009,6 +1087,7 @@ int wdpm_apply_add(wdpm_solver* s, double depth, double runoff_fraction) {
         k_apply_add<float><<<grid, 256, 0, s->stream>>>(static_cast<float*>(s->w[s->cur]), static_cast<const float*>(s->dem), n,
                                                         (float)depth, (float)(depth * runoff_fraction));
     s->water_clean = false;
+    s->negzero_free = false;  // depth * runoff_fraction may be -0.0
     s->launches++;
     CUDA_TRY(cudaGetLastError());
     return WDPM_OK;
@@ -1027,6 +1106,7 @@ int wdpm_apply_subtract(wdpm_solver* s, double depth) {
         k_apply_subtract<float><<<grid, 256, 0, s->stream>>>(static_cast<float*>(s->w[s->cur]), static_cast<const float*>(s->dem), n,
                                                              (float)depth);
     s->water_clean = false;
+    s->negzero_free = true;  // every valid cell is now > 0 or +0
     s->launches++;
     CUDA_TRY(cudaGetLastError());
     return WDPM_OK;
@@ -1066,6 +1146,7 @@ int wdpm_set_outlets(wdpm_solver* s, int32_t n, const int32_t* rows, const int32
     if (!s || (n > 0 && (!rows || !cols))) return fail(WDPM_E_ARG, "null argument");
     if (s->module != WDPM_DRAIN) return fail(WDPM_E_STATE, "outlets belong to the Drain module");
     if (n < 1 || n > kMaxOutlets) return fail(WDPM_E_ARG, "number of outlets must be in 1..WDPM_MAX_OUTLETS");
+    if (n > 1 && s->schedule == WDPM_SCHEDULE_SERIAL) return fail(WDPM_E_UNSUPPORTED, "the serial schedule has one outlet (the emptying of overlapping outlet neighbourhoods is not defined)");
     if (s->in_block) return fail(WDPM_E_STATE, "a block is open");
     for (int k = 0; k < n; k++) {
         if (rows[k] < 0 || rows[k] > s->cfg.rows + 1 || cols[k] < 0 || cols[k] > s->g.C + 1) return fail(WDPM_E_ARG, "outlet outside the padded grid");
@@ -1142,6 +1223,7 @@ int wdpm_quantize_water(wdpm_solver* s) {
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaStreamSynchronize(s->stream));
     s->water_clean = false;
+    s->negzero_free = false;  // a tiny negative value quantises to -0.0
     return WDPM_OK;
 }
 

@@ -11,10 +11,12 @@
  * the water grid comes back only for a scratch file or the final output.
  *
  * The two backend selectors of the reference command line ("0 serial / 1 OpenCL",
- * "0 OpenCL CPU / 1 OpenCL GPU") are still parsed at their positions; whatever
- * they say, the CUDA solver runs - there is no CPU path - and the report says so.
- * The update schedule is the OpenCL branch's (runoff.cl arithmetic); see DESIGN.md
- * for how that differs from the serial branch in the last bits of Drain/Subtract.
+ * "0 OpenCL CPU / 1 OpenCL GPU") are parsed at their positions; whatever they say,
+ * the CUDA solver runs - there is no CPU path - and the report says so. The first
+ * picks the arithmetic, as it does in the reference, where the two branches differ
+ * in Subtract and Drain (DESIGN.md §4): "cpu" = 0 runs the serial branch's
+ * (WDPM_SCHEDULE_SERIAL), any other value the OpenCL branch's (runoff.cl). The
+ * second flag (OpenCL device kind) is ignored.
  *
  * Extension: `wdpmcl_b200 chain paramfile1 paramfile2 ...` runs several modules in ONE process (the
  * reference's validate_WDPM.sh:77-99 runs Add -> Drain -> Subtract as three). Each module prints its
@@ -187,9 +189,10 @@ static void echo_args(const run_args *a)
     else printf("%30s %d\n", "Maximum number of iterations:", a->iter_limit);
     line("               ");
     /* the reference prints which OpenCL/serial backend the two flags select (:1781-1796);
-     * here both flags select the same thing */
+     * here the first one selects the arithmetic only */
     printf("%41s\n", "Using CUDA (sm_100a) for Computation");
-    printf("%40s\n", "backend flags accepted and ignored");
+    if (a->backend == 0) printf("%40s\n", "serial-branch arithmetic on CUDA");
+    else printf("%40s\n", "backend flags accepted and ignored");
 }
 
 /* ---- arguments: positional argv or a whitespace-token parameter file ------- */
@@ -747,6 +750,7 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     cfg.dtype = WDPM_F64;
     cfg.module = is_add ? WDPM_ADD : is_sub ? WDPM_SUBTRACT : WDPM_DRAIN;
     cfg.zero_threshold = thres;
+    cfg.schedule = a.backend == 0 ? WDPM_SCHEDULE_SERIAL : WDPM_SCHEDULE_OPENCL;
     cfg.device = getenv("WDPM_B200_DEVICE") ? atoi(getenv("WDPM_B200_DEVICE")) : 0;
     cfg.kernel = getenv("WDPM_B200_KERNEL") ? atoi(getenv("WDPM_B200_KERNEL")) : WDPM_KERNEL_AUTO;
     solver_set ss;

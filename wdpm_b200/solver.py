@@ -16,6 +16,8 @@ import numpy as np
 ADD, SUBTRACT, DRAIN = 0, 1, 2
 F32, F64 = 0, 1
 KERNEL_AUTO, KERNEL_COLOUR, KERNEL_FUSED, KERNEL_RESIDENT = 0, 1, 2, 3
+# update schedule (WDPM_SCHEDULE_* in include/wdpm_b200.h): the reference's OpenCL branch, or its serial branch
+SCHED_OPENCL, SCHED_SERIAL = 0, 1
 MODULES = {"add": ADD, "subtract": SUBTRACT, "drain": DRAIN}
 # the tiling AUTO picks for large fp64 Add/Subtract grids (kDefaultVariantF64 in csrc/solver.cu); tests and
 # smoke() name it to exercise the production kernel on small grids
@@ -36,7 +38,7 @@ class _Config(C.Structure):
                 ("dtype", C.c_int32), ("module", C.c_int32), ("zero_threshold", C.c_double), ("device", C.c_int32),
                 ("kernel", C.c_int32), ("stripe_row0", C.c_int32), ("stripe_rows", C.c_int32),
                 ("iters_per_launch", C.c_int32), ("fused_variant", C.c_int32), ("fused_chunk_rows", C.c_int32),
-                ("reserved", C.c_int32 * 5)]
+                ("schedule", C.c_int32), ("reserved", C.c_int32 * 4)]
 
 
 class _BlockResult(C.Structure):
@@ -110,7 +112,7 @@ class Solver:
 
     def __init__(self, rows: int, cols: int, nodata: float, module: int, dtype: int = F64, zero_threshold: float = 0.0,
                  device: int = 0, kernel: int = KERNEL_AUTO, iters_per_launch: int = 0, fused_variant: int = 0,
-                 fused_chunk_rows: int = 0, _stripe: tuple | None = None):
+                 fused_chunk_rows: int = 0, schedule: int = SCHED_OPENCL, _stripe: tuple | None = None):
         self._lib = load_library()
         self._h = C.c_void_p()
         cfg = _Config()
@@ -120,8 +122,10 @@ class Solver:
         cfg.device, cfg.kernel = device, kernel
         cfg.stripe_row0, cfg.stripe_rows = _stripe if _stripe else (0, 0)
         cfg.iters_per_launch, cfg.fused_variant, cfg.fused_chunk_rows = iters_per_launch, fused_variant, fused_chunk_rows
+        cfg.schedule = schedule
         _check(self._lib.wdpm_create(C.byref(cfg), C.byref(self._h)))
         self.rows, self.cols, self.dtype, self.module, self.nodata = rows, cols, dtype, module, nodata
+        self.schedule = schedule
         self.np_dtype = _np_dtype(dtype)
 
     # -- lifetime ---------------------------------------------------------
