@@ -147,14 +147,24 @@ int wdpm_set_outlet(wdpm_solver *s, int32_t drainrow, int32_t draincol);
  * (solver precision). Replaces any earlier set. Drain solvers only. Row stripes: every stripe is given the whole
  * set; an outlet's total is kept by the stripe that owns its row - contacts from centres of a neighbouring stripe
  * are recorded there too, in sub-pass order, so each total is bit-identical to the single-GPU one - and reads as 0 on
- * the other stripes: a host adds the stripes' wdpm_get_outlet_drains element by element. */
-#define WDPM_MAX_OUTLETS 1024
+ * the other stripes: a host adds the stripes' wdpm_get_outlet_drains element by element.
+ * Up to WDPM_MAX_OUTLETS cells, each inside the DEM (row 1..rows, col 1..cols) and on a cell with dem > nodata;
+ * otherwise, and for a duplicate, WDPM_E_ARG. The dem test runs once the set and an uploaded DEM meet (here, or
+ * in a later upload, which then fails and leaves no set installed). The serial schedule refuses a set of more than one
+ * outlet (WDPM_E_UNSUPPORTED). The solver sorts the set; the time a kernel spends on an outlet contact grows as
+ * log2(n), and the device memory the set takes grows linearly in n (DESIGN.md section 3.3 gives the bound).
+ * wdpm_get_outlet_drains returns the first n totals in the caller's order (n at most the set's size). */
+#define WDPM_MAX_OUTLETS 1048576
 int wdpm_set_outlets(wdpm_solver *s, int32_t n, const int32_t *rows, const int32_t *cols);
 int wdpm_get_outlet_drains(wdpm_solver *s, double *values, int32_t n);
 /* totaldrain accumulator (src/WDPMCL.c:1029, :1136); with an outlet set, set writes the first
- * outlet's total and zeroes the others, get returns the sum */
+ * outlet's total and zeroes the others, get returns the sum (computed on the device) */
 int wdpm_set_total_drain(wdpm_solver *s, double value);
 int wdpm_get_total_drain(wdpm_solver *s, double *value);
+/* Seed every outlet's total with max(water at the outlet, 0): src/WDPMCL.c:1029 applied to each outlet. On row
+ * stripes the stripe that owns the outlet's row does it and the others set 0. For one outlet it equals
+ * wdpm_get_cell_water followed by wdpm_set_total_drain(max(w, 0)). */
+int wdpm_seed_outlet_drains(wdpm_solver *s);
 /* Module chaining. The reference runs Add -> Drain -> Subtract as three processes that hand the
  * water grid on through "%f" text files (validation/validate_WDPM.sh:77-99). A host that runs the
  * modules in one process can keep the grids in HBM instead:

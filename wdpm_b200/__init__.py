@@ -5,9 +5,9 @@ include/wdpm_b200.h) and the drop-in command-line host (host/). The Python
 modules here are a thin ctypes mirror of that ABI plus the module driver used by
 the tests and the benchmark.
 """
-from .solver import (ADD, DRAIN, F32, F64, KERNEL_AUTO, KERNEL_COLOUR, KERNEL_FUSED, KERNEL_RESIDENT, SCHED_OPENCL, SCHED_SERIAL, SUBTRACT,
+from .solver import (ADD, DRAIN, F32, F64, MAX_OUTLETS, KERNEL_AUTO, KERNEL_COLOUR, KERNEL_FUSED, KERNEL_RESIDENT, SCHED_OPENCL, SCHED_SERIAL, SUBTRACT,
                      BlockResult, Solver, WdpmError, library_path, load_library)
 
 __all__ = ["ADD", "SUBTRACT", "DRAIN", "F32", "F64", "KERNEL_AUTO", "KERNEL_COLOUR", "KERNEL_FUSED", "KERNEL_RESIDENT", "SCHED_OPENCL",
-           "SCHED_SERIAL", "BlockResult",
+           "SCHED_SERIAL", "MAX_OUTLETS", "BlockResult",
            "Solver", "WdpmError", "library_path", "load_library"]

@@ -71,6 +71,16 @@ def write_asc(path, hdr: AscHeader, grid: np.ndarray) -> None:
     Path(path).write_text(out.getvalue())
 
 
+def rim_outlets(dem: np.ndarray, nodata: float) -> list[tuple[int, int]]:
+    """The outlet set "rim" of the command-line host (WDPM_B200_OUTLETS=rim): every cell with dem > nodata in the
+    first or last row or column of the (unpadded) DEM, in row-major order, as 1-based padded (row, col)."""
+    R, C = dem.shape
+    on_rim = np.zeros((R, C), dtype=bool)
+    on_rim[0, :] = on_rim[-1, :] = on_rim[:, 0] = on_rim[:, -1] = True
+    r, c = np.nonzero(on_rim & (dem > nodata))
+    return list(zip((r + 1).tolist(), (c + 1).tolist()))
+
+
 def pad_grid(a: np.ndarray, fill) -> np.ndarray:
     """(R, C) -> (R+2, C+2) with a one-cell border of `fill` (WDPMCL.c:795-807)."""
     out = np.full((a.shape[0] + 2, a.shape[1] + 2), fill, dtype=a.dtype)

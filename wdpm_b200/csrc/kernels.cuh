@@ -304,14 +304,14 @@ __global__ void k_find_outlet_stage2(const OutletCand* __restrict__ partials, in
 // the reference's totaldrain, src/runoff.cl:108). An event is the pair of addends of one outlet
 // contact, folded as (total + w_outlet) + w_centre, in sub-pass order. An outlet is a neighbour of
 // at most one centre per colour sub-pass, so (outlet, sub-pass) identifies a contact.
+// The set is sorted by (row, col) when it is installed (solver.cu); kernels find an outlet by binary search
+// and keep its total at its sorted position.
 // ---------------------------------------------------------------------------
 
 template <typename T>
-struct DrainEvent {
+struct DrainPair {
     T w_outlet;
     T w_centre;
-    int valid;
-    int pad;
 };
 
 // Event buffers rotate over kEventSlots launches: launch L records into buffer L % 3 and folds buffer (L-1) % 3.
@@ -325,68 +325,194 @@ constexpr int kEventSlots = 3;
 __host__ __device__ __forceinline__ int next_event_slot(int s) { return s == kEventSlots - 1 ? 0 : s + 1; }
 __host__ __device__ __forceinline__ int prev_event_slot(int s) { return s == 0 ? kEventSlots - 1 : s - 1; }
 
-template <typename T>
-struct DrainState {
-    T* totaldrain;          // [n_outlets] device accumulators
-    DrainEvent<T>* events;  // [kEventSlots][n_outlets][9*kMaxItersPerLaunch]
-    const int* outlet_rc;   // [n_outlets][2] padded (row, col) of each outlet in this solver's rows
-    int n_outlets;
-    // row stripes: the event buffers of the stripes above / below (peer memory; nullptr = none) and this stripe's owned rows
-    DrainEvent<T>* events_up;
-    DrainEvent<T>* events_dn;
-    int P;
+// An event area: per buffer and entry a bit mask of the sub-pass slots that hold a contact, the addends of those
+// contacts at their slots, and the list of entries touched since the buffer was last folded. Recording sets a bit
+// (the first bit of an entry appends the entry to the list); folding walks the list only, so it costs time in
+// proportion to the outlets that were touched, not to the size of the set. Two areas exist:
+//  - the outlet area, one entry per outlet (sorted position), allocated when the set is installed;
+//  - row stripes only, the border area, one entry per column of the stripe's first and of its last owned row,
+//    allocated with the stripe's arrival flags (one IPC handle covers both; a neighbour records there the
+//    contacts of its centres with my outlets). Every contact with an outlet in one of those two rows goes there,
+//    whichever stripe's centre made it, so each outlet's events stay in one place.
+struct EventCounters {
+    int n_touched[kEventSlots];  // entries on each buffer's touched list
+    int fold_done[kEventSlots];  // thread groups that have folded the buffer (the last one empties the lists)
 };
 
-constexpr int kEventsPerBuffer = 9 * kMaxItersPerLaunch;
-
 template <typename T>
-__device__ __forceinline__ DrainEvent<T>* event_slot(DrainEvent<T>* events, int n_outlets, int buffer, int outlet, int slot) {
-    return events + ((size_t)buffer * n_outlets + outlet) * kEventsPerBuffer + slot;
+struct EventArea {
+    EventCounters* ctr;
+    unsigned long long* mask;  // [kEventSlots][n]
+    int* touched;              // [kEventSlots][n]
+    DrainPair<T>* vals;        // [kEventSlots][n][slots]
+    int n;                     // entries (0 = no area)
+    int slots;                 // sub-pass slots per entry and buffer: 9 per iteration of a launch, + 1 (kWipeSlot)
+};
+
+__host__ __device__ __forceinline__ size_t event_area_bytes(long long n, int slots, size_t esize) {
+    const size_t mask_off = 256, touched_off = mask_off + (size_t)kEventSlots * n * 8;
+    const size_t vals_off = (touched_off + (size_t)kEventSlots * n * 4 + 15) / 16 * 16;
+    return vals_off + (size_t)kEventSlots * n * slots * 2 * esize;
 }
 
-// index of the outlet at padded (row, col); -1 if none (cannot happen for a marked cell)
+template <typename T>
+__host__ __device__ __forceinline__ EventArea<T> event_area(void* base, int n, int slots) {
+    EventArea<T> a;
+    char* b = static_cast<char*>(base);
+    const size_t touched_off = 256 + (size_t)kEventSlots * n * 8;
+    a.ctr = reinterpret_cast<EventCounters*>(b);
+    a.mask = reinterpret_cast<unsigned long long*>(b + 256);
+    a.touched = reinterpret_cast<int*>(b + touched_off);
+    a.vals = reinterpret_cast<DrainPair<T>*>(b + (touched_off + (size_t)kEventSlots * n * 4 + 15) / 16 * 16);
+    a.n = base ? n : 0;
+    a.slots = slots;
+    return a;
+}
+
+template <typename T>
+struct DrainState {
+    T* totaldrain;          // [n_outlets] device accumulators, in sorted order
+    const int* outlet_rc;   // [n_outlets][2] padded (row, col) of each outlet in this solver's rows, sorted by (row, col)
+    int n_outlets;
+    EventArea<T> ev;        // outlet area
+    // row stripes: this stripe's border area and its neighbours' (peer memory; n = 0: none), and its owned rows
+    EventArea<T> border, border_up, border_dn;
+    int P;
+    int border_cols;        // entries per border row (cols + 2)
+    const unsigned char* cta_outlets;  // fused kernels: [CTA] 1 = an outlet lies in the rows and columns the CTA stages
+};
+
+// sorted position of the outlet at padded (row, col); -1 if none (cannot happen for a marked cell)
 template <typename T>
 __device__ __forceinline__ int outlet_index(const DrainState<T>& ds, int row, int col) {
-    for (int k = 0; k < ds.n_outlets; k++)
-        if (ds.outlet_rc[2 * k] == row && ds.outlet_rc[2 * k + 1] == col) return k;
-    return -1;
+    int lo = 0, hi = ds.n_outlets;  // first position whose (row, col) is not below the key
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        const int r = ds.outlet_rc[2 * mid], c = ds.outlet_rc[2 * mid + 1];
+        if (r < row || (r == row && c < col)) lo = mid + 1;
+        else hi = mid;
+    }
+    return (lo < ds.n_outlets && ds.outlet_rc[2 * lo] == row && ds.outlet_rc[2 * lo + 1] == col) ? lo : -1;
 }
 
-// Fold one event buffer: thread t of the calling group takes outlets t, t + nthreads, ...
+// Fold entries first, first + stride, ... of the touched list of `buffer` in area `a` into their outlets' totals,
+// slot by slot in sub-pass order.
 template <typename T>
-__device__ __forceinline__ void fold_events(const DrainState<T>& ds, int buffer, int t, int nthreads) {
-    for (int k = t; k < ds.n_outlets; k += nthreads) {
-        DrainEvent<T>* ev = event_slot(ds.events, ds.n_outlets, buffer, k, 0);
+__device__ __forceinline__ void fold_area(const DrainState<T>& ds, const EventArea<T>& a, bool border, int buffer, int first, int stride) {
+    const int n = *reinterpret_cast<volatile int*>(&a.ctr->n_touched[buffer]);
+    for (int i = first; i < n; i += stride) {
+        const int entry = a.touched[(size_t)buffer * a.n + i];
+        const size_t e = (size_t)buffer * a.n + entry;
+        unsigned long long m = a.mask[e];
+        a.mask[e] = 0ull;
+        const int k = border ? outlet_index(ds, entry < ds.border_cols ? 0 : ds.P - 1, entry % ds.border_cols) : entry;
+        if (k < 0) continue;
+        const DrainPair<T>* v = a.vals + e * a.slots;
         T td = ds.totaldrain[k];
-        bool any = false;
-        for (int e = 0; e < kEventsPerBuffer; e++) {
-            if (ev[e].valid) {
-                td = td + ev[e].w_outlet;
-                td = td + ev[e].w_centre;
-                ev[e].valid = 0;
-                any = true;
-            }
+        while (m) {
+            const int s = __ffsll((long long)m) - 1;
+            m &= m - 1;
+            td = td + v[s].w_outlet;
+            td = td + v[s].w_centre;
         }
-        if (any) ds.totaldrain[k] = td;
+        ds.totaldrain[k] = td;
+    }
+}
+
+// Fold one event buffer: the calling threads split the touched entries (thread `first` of `stride`). Every group
+// of threads that takes part must then call fold_finish once, after a barrier over the group.
+template <typename T>
+__device__ __forceinline__ void fold_events(const DrainState<T>& ds, int buffer, int first, int stride) {
+    fold_area(ds, ds.ev, false, buffer, first, stride);
+    if (ds.border.n) fold_area(ds, ds.border, true, buffer, first, stride);
+}
+
+// One thread per group that folded `buffer` (`groups` of them): the last to arrive empties the touched lists.
+template <typename T>
+__device__ __forceinline__ void fold_finish(const DrainState<T>& ds, int buffer, int groups) {
+    if (atomicAdd(&ds.ev.ctr->fold_done[buffer], 1) == groups - 1) {
+        ds.ev.ctr->n_touched[buffer] = 0;
+        if (ds.border.n) ds.border.ctr->n_touched[buffer] = 0;
+        ds.ev.ctr->fold_done[buffer] = 0;
     }
 }
 
 template <typename T>
 __global__ void k_fold_events(DrainState<T> ds, int buffer) {
-    if (blockIdx.x == 0) fold_events(ds, buffer, (int)threadIdx.x, (int)blockDim.x);
+    fold_events(ds, buffer, (int)(blockIdx.x * blockDim.x + threadIdx.x), (int)(gridDim.x * blockDim.x));
+    __syncthreads();
+    if (threadIdx.x == 0) fold_finish(ds, buffer, (int)gridDim.x);
 }
 
 // Mark / unmark outlet cells in the elevation grid (relax.cuh, outlet_mark). `saved` keeps the
-// elevations the marks replace so they can be restored (module change, new outlet set).
+// elevations the marks replace so they can be restored (module change, new outlet set). Marking also counts in
+// `bad` the outlets on cells of local rows [data_lo, data_hi) (the rows that hold DEM data) with dem <= nodata.
 template <typename T>
-__global__ void k_mark_outlets(T* __restrict__ d, Geom g, const int* __restrict__ rc, int n, T* __restrict__ saved, int restore) {
+__global__ void k_mark_outlets(T* __restrict__ d, Geom g, const int* __restrict__ rc, int n, T* __restrict__ saved, int restore,
+                               int data_lo, int data_hi, int* __restrict__ bad) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
     const int i = rc[2 * k], j = rc[2 * k + 1];
     if (i < -kPadTop || i >= g.nrows_dev - kPadTop || j < 0 || j > g.C + 1) return;  // not in this solver's rows
     const size_t a = dev_index(g, i, j);
-    if (restore) d[a] = saved[k];
-    else { saved[k] = d[a]; d[a] = outlet_mark<T>(); }
+    if (restore) {
+        d[a] = saved[k];
+    } else {
+        if (i >= data_lo && i < data_hi && !is_valid_elevation(d[a])) atomicAdd(bad, 1);
+        saved[k] = d[a];
+        d[a] = outlet_mark<T>();
+    }
+}
+
+// Totals seeded from the water under the outlets (src/WDPMCL.c:1029 per outlet): max(w, 0) where this solver owns
+// the outlet's row, 0 elsewhere.
+template <typename T>
+__global__ void k_seed_outlets(const T* __restrict__ w, Geom g, DrainState<T> ds) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= ds.n_outlets) return;
+    const int i = ds.outlet_rc[2 * k], j = ds.outlet_rc[2 * k + 1];
+    T v = T(0);
+    if (i >= 0 && i < ds.P) {
+        const T x = w[dev_index(g, i, j)];
+        v = x > T(0) ? x : T(0);
+    }
+    ds.totaldrain[k] = v;
+}
+
+// The reported total: the outlets' totals added in the caller's order, in the solver's precision. One thread:
+// the order is the definition (an outlet-order sum of the host-side totals gives the same bits).
+template <typename T>
+__global__ void k_sum_totals(const T* __restrict__ totals, const int* __restrict__ pos, int n, double* __restrict__ out) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    T t = totals[pos[0]];
+    for (int k = 1; k < n; k++) t = t + totals[pos[k]];
+    *out = (double)t;
+}
+
+// Record one event: its addends go into slot `slot` of `entry` in buffer `buffer` of area `a`. `sys`: a border
+// area, into which the neighbour's centres record from another GPU too (system-scope atomics); only this solver's
+// kernels write its outlet area.
+template <typename T>
+__device__ __forceinline__ void record_event(const EventArea<T>& a, int buffer, int entry, int slot, T w_outlet, T w_centre, bool sys) {
+    const size_t e = (size_t)buffer * a.n + entry;
+    DrainPair<T>* v = a.vals + e * a.slots + slot;
+    v->w_outlet = w_outlet;
+    v->w_centre = w_centre;
+    const unsigned long long bit = 1ull << slot;
+    const bool first = (sys ? atomicOr_system(&a.mask[e], bit) : atomicOr(&a.mask[e], bit)) == 0ull;
+    if (first) a.touched[(size_t)buffer * a.n + (sys ? atomicAdd_system(&a.ctr->n_touched[buffer], 1) : atomicAdd(&a.ctr->n_touched[buffer], 1))] = entry;
+}
+
+// Where the events of the outlet at local padded (orow, ocol) go: a border area (row stripes: the outlet's row is
+// the first or last owned row of this stripe or of a neighbour) or the outlet area.
+template <typename T>
+__device__ __forceinline__ void route_event(const DrainState<T>& ds, int buffer, int slot, int orow, int ocol, T w_outlet, T w_centre) {
+    if (ds.border_up.n && orow < 0) { record_event(ds.border_up, buffer, ds.border_cols + ocol, slot, w_outlet, w_centre, true); return; }
+    if (ds.border_dn.n && orow >= ds.P) { record_event(ds.border_dn, buffer, ocol, slot, w_outlet, w_centre, true); return; }
+    if (ds.border.n && orow == 0) { record_event(ds.border, buffer, ocol, slot, w_outlet, w_centre, true); return; }
+    if (ds.border.n && orow == ds.P - 1) { record_event(ds.border, buffer, ds.border_cols + ocol, slot, w_outlet, w_centre, true); return; }
+    const int k = outlet_index(ds, orow, ocol);
+    if (k >= 0) record_event(ds.ev, buffer, k, slot, w_outlet, w_centre, false);
 }
 
 // Record one contact of a centre with the outlet at padded (orow, ocol): its two addends go into slot
@@ -395,22 +521,16 @@ __global__ void k_mark_outlets(T* __restrict__ d, Geom g, const int* __restrict_
 // them to the total at once.
 template <typename T>
 __device__ __forceinline__ void record_contact(const DrainState<T>& ds, int buffer, int slot, int orow, int ocol, T w_outlet, T w_centre, bool direct) {
-    const int k = outlet_index(ds, orow, ocol);
-    if (k < 0) return;
     if (direct) {
+        const int k = outlet_index(ds, orow, ocol);
+        if (k < 0) return;
         T td = ds.totaldrain[k];
         td = td + w_outlet;
         td = td + w_centre;
         ds.totaldrain[k] = td;
         return;
     }
-    DrainEvent<T>* base = ds.events;
-    if (ds.events_up && orow < 0) base = ds.events_up;
-    else if (ds.events_dn && orow >= ds.P) base = ds.events_dn;
-    DrainEvent<T>* ev = event_slot(base, ds.n_outlets, buffer, k, slot);
-    ev->w_outlet = w_outlet;
-    ev->w_centre = w_centre;
-    ev->valid = 1;
+    route_event(ds, buffer, slot, orow, ocol, w_outlet, w_centre);
 }
 
 // ---------------------------------------------------------------------------
@@ -423,8 +543,7 @@ __device__ __forceinline__ void record_contact(const DrainState<T>& ds, int buff
 // (total + got) + 0 == total + got, because total + got is never -0.0 (got >= +0).
 // ---------------------------------------------------------------------------
 
-constexpr int kWipeSlot = 9;
-static_assert(kWipeSlot < kEventsPerBuffer, "the wipe event follows the nine sub-pass slots of one iteration");
+constexpr int kWipeSlot = 9;  // an area's slots per entry are 9 * iterations per launch + 1 > kWipeSlot
 
 template <typename T>
 __device__ __forceinline__ T outlet_wipe_sum(const T* w, const T* d, size_t pitch) {
@@ -451,10 +570,7 @@ __global__ void k_outlet_wipe(T* __restrict__ w, const T* __restrict__ d, Geom g
         if (direct) {
             ds.totaldrain[0] = ds.totaldrain[0] + got;
         } else {
-            DrainEvent<T>* ev = event_slot(ds.events, ds.n_outlets, buffer, 0, kWipeSlot);
-            ev->w_outlet = got;
-            ev->w_centre = T(0);
-            ev->valid = 1;
+            route_event(ds, buffer, kWipeSlot, orow, ocol, got, T(0));
         }
     }
     for (int i = orow - 1; i <= orow + 1; i++)
@@ -873,24 +989,19 @@ k_fused(const FusedParams<T> p) {
     MwTile<CFG> tile;
     tile.init(strip, chunk, p.chunk_triples, p.total_triples);
 
-    if (MODULE == kDrain && blockIdx.x == 0) fold_events(p.ds, prev_event_slot(p.launch_slot), tid, NALL);
+    // Drain: every CTA folds its share of the previous launch's contacts (the touched entries of its event buffer)
+    if (MODULE == kDrain) fold_events(p.ds, prev_event_slot(p.launch_slot), (int)blockIdx.x * NALL + tid, (int)gridDim.x * NALL);
 
     // Drain: does any outlet lie in the rows and columns this CTA stages? (If not, no tile of this CTA
-    // can see an outlet mark and the per-tile test is skipped.)
+    // can see an outlet mark and the per-tile test is skipped.) Worked out per CTA when the set is installed.
     __shared__ int s_cta_has_outlets;
     if (tid == 0) {
         for (int i = 0; i < NSTAGE; i++) mbar_init(&bars[i], 1);
         fence_mbar_init();
-        s_cta_has_outlets = 0;
+        s_cta_has_outlets = MODULE == kDrain ? p.ds.cta_outlets[blockIdx.x] : 0;
     }
     __syncthreads();
-    if (MODULE == kDrain) {
-        for (int k = tid; k < p.ds.n_outlets; k += NALL) {
-            const int orow = p.ds.outlet_rc[2 * k], ocol = p.ds.outlet_rc[2 * k + 1];
-            if (orow >= 3 * tile.m_lo && orow <= 3 * tile.m_hi + 2 && ocol >= tile.x0 && ocol < tile.x0 + W) s_cta_has_outlets = 1;
-        }
-        __syncthreads();
-    }
+    if (MODULE == kDrain && tid == 0) fold_finish(p.ds, prev_event_slot(p.launch_slot), (int)gridDim.x);
     const bool cta_has_outlets = MODULE == kDrain && s_cta_has_outlets != 0;
 
     // Barriers. The colour sub-steps of a step only order tiles of the SAME row triple (they exchange
@@ -1124,25 +1235,20 @@ k_fused_wa(const FusedParams<T> p) {
     MwTile<CFG> tile;
     tile.init(strip, chunk, p.chunk_triples, p.total_triples);
 
-    if (MODULE == kDrain && blockIdx.x == 0) fold_events(p.ds, prev_event_slot(p.launch_slot), tid, NALL);
+    // Drain: every CTA folds its share of the previous launch's contacts (the touched entries of its event buffer)
+    if (MODULE == kDrain) fold_events(p.ds, prev_event_slot(p.launch_slot), (int)blockIdx.x * NALL + tid, (int)gridDim.x * NALL);
 
     // Drain: does any outlet lie in the rows and columns this CTA stages? (If not, no window of this CTA can hold an
-    // outlet mark and the per-step test is skipped.)
+    // outlet mark and the per-step test is skipped.) Worked out per CTA when the set is installed.
     __shared__ int s_cta_has_outlets;
     if (tid == 0) {
         for (int i = 0; i < NSTAGE; i++) mbar_init(&bars[i], 1);
         for (int i = 0; i < NPH * NT; i++) mbar_init(&group_bars[i], KW);
         fence_mbar_init();
-        s_cta_has_outlets = 0;
+        s_cta_has_outlets = MODULE == kDrain ? p.ds.cta_outlets[blockIdx.x] : 0;
     }
     __syncthreads();
-    if (MODULE == kDrain) {
-        for (int k = tid; k < p.ds.n_outlets; k += NALL) {
-            const int orow = p.ds.outlet_rc[2 * k], ocol = p.ds.outlet_rc[2 * k + 1];
-            if (orow >= 3 * tile.m_lo && orow <= 3 * tile.m_hi + 2 && ocol >= tile.x0 && ocol < tile.x0 + W) s_cta_has_outlets = 1;
-        }
-        __syncthreads();
-    }
+    if (MODULE == kDrain && tid == 0) fold_finish(p.ds, prev_event_slot(p.launch_slot), (int)gridDim.x);
     const bool cta_has_outlets = MODULE == kDrain && s_cta_has_outlets != 0;
 
     if (tid >= NTHREADS) {
@@ -1362,20 +1468,24 @@ k_resident(const ResidentParams<T> p) {
     const bool wipe = MODULE == kDrain && p.serial_wipe;
     const int orow = wipe ? p.ds.outlet_rc[0] : 0, ocol = wipe ? p.ds.outlet_rc[1] : 0;
     const bool wipe_owner = wipe && orow >= r_own && orow < r_own + p.TR && ocol >= c_own && ocol < c_own + p.TC;
-    const bool folder = wipe ? wipe_owner : blockIdx.x == 0;
+    // Otherwise every CTA folds its share of the previous iteration's contacts.
+    const bool fold_all = MODULE == kDrain && !wipe;
+    const int fold_first = (int)blockIdx.x * NTHREADS + tid, fold_stride = (int)gridDim.x * NTHREADS;
     int cur = p.cur, evbuf = p.launch_slot;
     for (int it = 0; it < p.n_iters; it++) {
         const T* __restrict__ win = p.w[cur];
         T* __restrict__ wout = p.w[cur ^ 1];
-        if (MODULE == kDrain && folder && !wipe) fold_events(p.ds, prev_event_slot(evbuf), tid, NTHREADS);
+        if (fold_all) fold_events(p.ds, prev_event_slot(evbuf), fold_first, fold_stride);
         for (int k = tid; k < SR * SC; k += NTHREADS) {
             const int i = k / SC, j = k - i * SC;
             sw[k] = win[base + (size_t)i * pitch + j];
         }
         __syncthreads();
+        if (fold_all && tid == 0) fold_finish(p.ds, prev_event_slot(evbuf), (int)gridDim.x);
         if (wipe) {
             if (wipe_owner && tid == 0) {
                 fold_events(p.ds, prev_event_slot(evbuf), 0, 1);
+                fold_finish(p.ds, prev_event_slot(evbuf), 1);
                 if (it > 0) {  // the launch before ended with its own emptying
                     const int a = (orow - r0) * SC + (ocol - c0);
                     p.ds.totaldrain[0] = p.ds.totaldrain[0] + outlet_wipe_sum(sw + a, sd + a, (size_t)SC);
@@ -1420,9 +1530,14 @@ k_resident(const ResidentParams<T> p) {
         cur ^= 1;
         evbuf = next_event_slot(evbuf);
     }
-    if (MODULE == kDrain && folder && !wipe) fold_events(p.ds, prev_event_slot(evbuf), tid, NTHREADS);
+    if (fold_all) {
+        fold_events(p.ds, prev_event_slot(evbuf), fold_first, fold_stride);
+        __syncthreads();
+        if (tid == 0) fold_finish(p.ds, prev_event_slot(evbuf), (int)gridDim.x);
+    }
     if (wipe_owner && tid == 0 && p.n_iters > 0) {
         fold_events(p.ds, prev_event_slot(evbuf), 0, 1);
+        fold_finish(p.ds, prev_event_slot(evbuf), 1);
         T* w = p.w[cur];
         const size_t c = dev_index(p.g, orow, ocol);
         p.ds.totaldrain[0] = p.ds.totaldrain[0] + outlet_wipe_sum(w + c, p.dem + c, pitch);

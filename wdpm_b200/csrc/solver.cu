@@ -262,12 +262,21 @@ struct wdpm_solver {
     bool negzero_free = false;
     int* d_dirty = nullptr;   // device flag of k_check_invalid_water
 
-    // Drain outlets (kernels.cuh "Drain bookkeeping"): capacity kMaxOutlets
-    void* totaldrain = nullptr;    // T[kMaxOutlets] per-outlet accumulators
-    void* events = nullptr;        // DrainEvent<T>[2][n_outlets][kEventsPerBuffer]
-    void* saved_elev = nullptr;    // T[kMaxOutlets] elevations under the outlet marks
-    int* d_outlet_rc = nullptr;    // int[kMaxOutlets][2] padded (row, col), rows local to this solver
+    // Drain outlets (kernels.cuh "Drain bookkeeping"). The per-outlet arrays hold outlet_cap entries: the installed
+    // set's size (1 before any set, so that the single total exists).
+    int outlet_cap = 0;
+    void* totaldrain = nullptr;    // T[outlet_cap] per-outlet accumulators, sorted order
+    void* ev_area = nullptr;       // the outlet event area (kernels.cuh, EventArea) for outlet_cap entries
+    int ev_slots = 10;             // its sub-pass slots per entry: 9 * iterations per launch + 1
+    void* events = nullptr;        // row stripes (Drain): the border event area, after the arrival flags; nullptr otherwise
+    void* saved_elev = nullptr;    // T[outlet_cap] elevations under the outlet marks
+    int* d_outlet_rc = nullptr;    // int[outlet_cap][2] padded (row, col), rows local to this solver, sorted by (row, col)
+    int* d_outlet_pos = nullptr;   // int[outlet_cap]: sorted position of the caller's outlet k
+    unsigned char* d_cta_outlets = nullptr;  // fused kernels: per CTA, does an outlet lie in what it stages
+    double* d_total = nullptr;     // the outlet-order sum of the totals (k_sum_totals)
+    int* d_bad = nullptr;          // outlets found on cells with dem <= nodata (k_mark_outlets)
     std::vector<int> outlet_rc;    // host copy of d_outlet_rc
+    std::vector<int> outlet_pos;   // host copy of d_outlet_pos
     int n_outlets = 0;
     bool marks_applied = false;
     bool have_outlet = false;
@@ -311,17 +320,23 @@ struct wdpm_solver {
 
 namespace {
 
+int border_entries(const wdpm_solver* s) { return 2 * (s->g.C + 2); }
+
 template <typename T>
 DrainState<T> drain_state(wdpm_solver* s) {
     DrainState<T> ds;
     ds.totaldrain = static_cast<T*>(s->totaldrain);
-    ds.events = static_cast<DrainEvent<T>*>(s->events);
     ds.outlet_rc = s->d_outlet_rc;
     ds.n_outlets = s->n_outlets;
-    // row stripes: contacts with an outlet in a neighbour's rows are recorded in that neighbour's buffer (kernels.cuh)
-    ds.events_up = (s->stripe && s->above.present) ? static_cast<DrainEvent<T>*>(s->above.events) : nullptr;
-    ds.events_dn = (s->stripe && s->below.present) ? static_cast<DrainEvent<T>*>(s->below.events) : nullptr;
+    ds.ev = event_area<T>(s->ev_area, s->outlet_cap, s->ev_slots);
+    // row stripes: contacts with an outlet in the first or last owned row of a stripe are recorded in that stripe's
+    // border area, a neighbour's over NVLink (kernels.cuh)
+    ds.border = event_area<T>(s->events, border_entries(s), s->ev_slots);
+    ds.border_up = event_area<T>((s->stripe && s->above.present) ? s->above.events : nullptr, border_entries(s), s->ev_slots);
+    ds.border_dn = event_area<T>((s->stripe && s->below.present) ? s->below.events : nullptr, border_entries(s), s->ev_slots);
     ds.P = s->P;
+    ds.border_cols = s->g.C + 2;
+    ds.cta_outlets = s->d_cta_outlets;
     return ds;
 }
 
@@ -345,7 +360,13 @@ int outlet_wipe(wdpm_solver* s, bool direct) {
 }
 
 constexpr int kMaxOutlets = WDPM_MAX_OUTLETS;
-constexpr size_t kFlagsBytes = 256;  // HaloFlags, padded; the drain event buffers follow in the same allocation
+constexpr size_t kFlagsBytes = 256;  // HaloFlags, padded; a Drain stripe's border event area follows in the same allocation
+
+// grid of the event fold: enough threads for the touched entries (at most the area's entries)
+int fold_grid(const wdpm_solver* s) {
+    const long long n = (long long)s->outlet_cap + (s->events ? border_entries(s) : 0);
+    return (int)std::min<long long>((n + 255) / 256, (long long)s->sm_count * 4);
+}
 
 int grid_for(long long n, int threads, int sm_count) {
     long long b = (n + threads - 1) / threads;
@@ -471,7 +492,7 @@ int fused_iterations(wdpm_solver* s, int n) {
             const int rc = outlet_wipe<T>(s, false);
             if (rc) return rc;
         }
-        k_fold_events<T><<<1, 256, 0, s->stream>>>(drain_state<T>(s), prev_event_slot(s->launch_slot));
+        k_fold_events<T><<<fold_grid(s), 256, 0, s->stream>>>(drain_state<T>(s), prev_event_slot(s->launch_slot));
         s->launches++;
         CUDA_TRY(cudaGetLastError());
     }
@@ -512,7 +533,7 @@ int fold_last_launch(wdpm_solver* s) {
         const int rc = outlet_wipe<T>(s, false);
         if (rc) return rc;
     }
-    k_fold_events<T><<<1, 256, 0, s->stream>>>(drain_state<T>(s), prev_event_slot(s->launch_slot));
+    k_fold_events<T><<<fold_grid(s), 256, 0, s->stream>>>(drain_state<T>(s), prev_event_slot(s->launch_slot));
     s->launches++;
     CUDA_TRY(cudaGetLastError());
     return WDPM_OK;
@@ -630,8 +651,12 @@ int block_end_t(wdpm_solver* s, wdpm_block_result* out) {
     s->launches += 2;
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(s->h_result, s->d_result, sizeof(BlockPartial), cudaMemcpyDeviceToHost, s->stream));
-    std::vector<T> tds((size_t)(s->n_outlets > 0 ? s->n_outlets : 1), T(0));
-    CUDA_TRY(cudaMemcpyAsync(tds.data(), s->totaldrain, sizeof(T) * tds.size(), cudaMemcpyDeviceToHost, s->stream));
+    // one outlet: the reference's totaldrain; a set: summed in outlet order, solver precision, on the device
+    k_sum_totals<T><<<1, 32, 0, s->stream>>>(static_cast<const T*>(s->totaldrain), s->d_outlet_pos, std::max(s->n_outlets, 1), s->d_total);
+    s->launches++;
+    CUDA_TRY(cudaGetLastError());
+    double td = 0.0;
+    CUDA_TRY(cudaMemcpyAsync(&td, s->d_total, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
     if (s->stripe) CUDA_TRY(cudaMemcpyAsync(s->h_halo_error, &s->flags->error, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
     int dirty = 1;
     CUDA_TRY(cudaMemcpyAsync(&dirty, s->d_dirty, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
@@ -643,14 +668,12 @@ int block_end_t(wdpm_solver* s, wdpm_block_result* out) {
         return fail(WDPM_E_HALO, "a neighbouring stripe's halo did not arrive in time (WDPM_B200_HALO_TIMEOUT_MS): the block's results are void; upload again");
     }
     s->invalid_dry = dirty == 0;  // as of this block's prologue; the kernels never put water on an invalid cell
-    T td = tds[0];  // one outlet: the reference's totaldrain; a set: summed in outlet order, solver precision
-    for (size_t k = 1; k < tds.size(); k++) td = td + tds[k];
     s->in_block = false;
     if (out) {
         out->max_diff = s->h_result->max_diff;
         out->masked_sum = s->h_result->sum;
         out->wet_cells = (int64_t)s->h_result->wet;
-        out->total_drain = (double)td;
+        out->total_drain = td;
         out->iterations = s->blk_iters;
         out->launches = (int32_t)(s->launches - s->blk_launches0);
         CUDA_TRY(cudaEventElapsedTime(&out->block_ms, s->ev[0], s->ev[3]));
@@ -716,17 +739,85 @@ void choose_chunks(wdpm_solver* s, int K, int NT, int minb, int forced_rows) {
 }
 
 // Put the outlet marks into the elevation grid (on = true) or take them out again, restoring the
-// elevations they replaced (kernels.cuh, k_mark_outlets). Idempotent.
+// elevations they replaced (kernels.cuh, k_mark_outlets). Idempotent. An outlet on a cell with dem <= nodata in the
+// rows this solver holds DEM data for uninstalls the set and returns WDPM_E_ARG: the mark would make that cell count
+// as valid in the block reductions.
 int apply_outlet_marks(wdpm_solver* s, bool on) {
     if (s->n_outlets == 0 || s->marks_applied == on) return WDPM_OK;
     const int n = s->n_outlets, blocks = (n + 127) / 128;
+    // local rows with DEM data: the interior rows of the band a stripe was given (owned rows + halos)
+    const int data_lo = std::max(s->G - kHaloAbove, 1) - s->G, data_hi = std::min(s->G + s->P + kHaloBelow, s->cfg.rows + 1) - s->G;
+    if (on) CUDA_TRY(cudaMemsetAsync(s->d_bad, 0, sizeof(int), s->stream));
     if (s->dtype == WDPM_F64)
-        k_mark_outlets<double><<<blocks, 128, 0, s->stream>>>(static_cast<double*>(s->dem), s->g, s->d_outlet_rc, n, static_cast<double*>(s->saved_elev), on ? 0 : 1);
+        k_mark_outlets<double><<<blocks, 128, 0, s->stream>>>(static_cast<double*>(s->dem), s->g, s->d_outlet_rc, n, static_cast<double*>(s->saved_elev), on ? 0 : 1,
+                                                              s->stripe ? data_lo : 1, s->stripe ? data_hi : s->g.R + 1, s->d_bad);
     else
-        k_mark_outlets<float><<<blocks, 128, 0, s->stream>>>(static_cast<float*>(s->dem), s->g, s->d_outlet_rc, n, static_cast<float*>(s->saved_elev), on ? 0 : 1);
+        k_mark_outlets<float><<<blocks, 128, 0, s->stream>>>(static_cast<float*>(s->dem), s->g, s->d_outlet_rc, n, static_cast<float*>(s->saved_elev), on ? 0 : 1,
+                                                             s->stripe ? data_lo : 1, s->stripe ? data_hi : s->g.R + 1, s->d_bad);
     s->launches++;
     CUDA_TRY(cudaGetLastError());
     s->marks_applied = on;
+    if (!on) return WDPM_OK;
+    int bad = 0;
+    CUDA_TRY(cudaMemcpyAsync(&bad, s->d_bad, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if (bad == 0) return WDPM_OK;
+    const int rc = apply_outlet_marks(s, false);
+    if (rc) return rc;
+    s->n_outlets = 0;
+    s->have_outlet = false;
+    return fail(WDPM_E_ARG, std::to_string(bad) + " outlet(s) on cells with dem <= nodata: the set is refused");
+}
+
+// (Re)allocate the per-outlet arrays for `cap` outlets; new arrays are zeroed.
+int alloc_outlets(wdpm_solver* s, int cap) {
+    if (cap == s->outlet_cap) return WDPM_OK;
+    const size_t ev_bytes = event_area_bytes(cap, s->ev_slots, s->esize);
+    const size_t old_bytes = s->outlet_cap ? event_area_bytes(s->outlet_cap, s->ev_slots, s->esize) + (size_t)s->outlet_cap * (2 * s->esize + 12) : 0;
+    void* ptrs[] = {s->totaldrain, s->ev_area, s->saved_elev, s->d_outlet_rc, s->d_outlet_pos};
+    for (void* p : ptrs)
+        if (p) cudaFree(p);
+    s->totaldrain = s->ev_area = s->saved_elev = nullptr;
+    s->d_outlet_rc = s->d_outlet_pos = nullptr;
+    s->device_bytes -= (long long)old_bytes;
+    s->outlet_cap = 0;
+    CUDA_TRY(cudaMalloc(&s->totaldrain, s->esize * cap));
+    CUDA_TRY(cudaMalloc(&s->ev_area, ev_bytes));
+    CUDA_TRY(cudaMalloc(&s->saved_elev, s->esize * cap));
+    CUDA_TRY(cudaMalloc((void**)&s->d_outlet_rc, sizeof(int) * 2 * cap));
+    CUDA_TRY(cudaMalloc((void**)&s->d_outlet_pos, sizeof(int) * cap));
+    CUDA_TRY(cudaMemsetAsync(s->totaldrain, 0, s->esize * cap, s->stream));
+    CUDA_TRY(cudaMemsetAsync(s->ev_area, 0, ev_bytes, s->stream));
+    CUDA_TRY(cudaMemsetAsync(s->d_outlet_pos, 0, sizeof(int) * cap, s->stream));
+    s->outlet_cap = cap;
+    s->device_bytes += (long long)(ev_bytes + (size_t)cap * (2 * s->esize + 12));
+    return WDPM_OK;
+}
+
+// Which CTAs of the fused kernels stage an outlet cell (kernels.cuh, k_fused / k_fused_wa: s_cta_has_outlets). A
+// CTA of strip st and chunk c stages padded columns [st*TWV - HL, st*TWV - HL + W) and the rows of triples
+// m_lo = c*chunk - K .. m_hi = min((c+1)*chunk, total) + 2K - 1 (mw_schedule.h, MwTile::init).
+template <typename T>
+int compute_cta_outlets(wdpm_solver* s) {
+    const FusedVariant<T>& v = fused_variants<T>()[s->variant];
+    const int top = v.wa ? 1 : v.K, bot = v.wa ? 2 : 2 * v.K;
+    const int ct = s->chunk_triples;
+    std::vector<unsigned char> flags((size_t)s->n_strips * s->n_chunks, 0);
+    for (int k = 0; k < s->n_outlets; k++) {
+        const int r = s->outlet_rc[2 * k], col = s->outlet_rc[2 * k + 1];
+        const int c_first = std::max(0, (r / 3 - bot - ct) / ct - 1), c_last = std::min(s->n_chunks - 1, (r / 3 + top) / ct + 1);
+        for (int c = c_first; c <= c_last; c++) {
+            const int m_lo = c * ct - top, m_hi = std::min((c + 1) * ct, s->total_triples) + bot - 1;
+            if (r < 3 * m_lo || r > 3 * m_hi + 2) continue;
+            const int st_first = std::max(0, (col + v.HL - v.W) / v.TWV), st_last = std::min(s->n_strips - 1, (col + v.HL) / v.TWV);
+            for (int st = st_first; st <= st_last; st++) {
+                const int x0 = st * v.TWV - v.HL;
+                if (col >= x0 && col < x0 + v.W) flags[(size_t)c * s->n_strips + st] = 1;
+            }
+        }
+    }
+    CUDA_TRY(cudaMemcpyAsync(s->d_cta_outlets, flags.data(), flags.size(), cudaMemcpyHostToDevice, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
     return WDPM_OK;
 }
 
@@ -946,15 +1037,17 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
         s->device_bytes += (long long)grid_bytes;
     }
     s->reduce_blocks = s->sm_count * 8;
-    // the arrival flags and the drain event buffers share one allocation: both are written by the neighbouring
-    // stripes, and one IPC handle then covers both
-    const size_t ev_bytes = (size_t)kEventSlots * kMaxOutlets * kEventsPerBuffer * (s->dtype == WDPM_F64 ? sizeof(DrainEvent<double>) : sizeof(DrainEvent<float>));
+    // the arrival flags and a Drain stripe's border event area share one allocation: both are written by the
+    // neighbouring stripes, and one IPC handle then covers both
+    s->ev_slots = 9 * K + 1;
+    const size_t ev_bytes = (is_stripe && cfg->module == WDPM_DRAIN) ? event_area_bytes(2 * (cfg->cols + 2), s->ev_slots, s->esize) : 0;
     if ((e = cudaMalloc((void**)&s->flags, kFlagsBytes + ev_bytes)) != cudaSuccess) return cleanup(WDPM_E_NOMEM, cudaGetErrorString(e));
-    s->events = reinterpret_cast<char*>(s->flags) + kFlagsBytes;
-    if ((e = cudaMalloc(&s->totaldrain, 8 * kMaxOutlets)) != cudaSuccess ||
-        (e = cudaMalloc(&s->saved_elev, 8 * kMaxOutlets)) != cudaSuccess ||
-        (e = cudaMalloc((void**)&s->d_outlet_rc, sizeof(int) * 2 * kMaxOutlets)) != cudaSuccess ||
-        (e = cudaMalloc((void**)&s->partials, sizeof(BlockPartial) * s->reduce_blocks)) != cudaSuccess ||
+    s->device_bytes += (long long)(kFlagsBytes + ev_bytes);
+    if (ev_bytes) s->events = reinterpret_cast<char*>(s->flags) + kFlagsBytes;
+    if ((e = cudaMalloc((void**)&s->partials, sizeof(BlockPartial) * s->reduce_blocks)) != cudaSuccess ||
+        (e = cudaMalloc((void**)&s->d_cta_outlets, (size_t)s->n_strips * s->n_chunks)) != cudaSuccess ||
+        (e = cudaMalloc((void**)&s->d_total, sizeof(double))) != cudaSuccess ||
+        (e = cudaMalloc((void**)&s->d_bad, sizeof(int))) != cudaSuccess ||
         (e = cudaMalloc((void**)&s->d_result, sizeof(BlockPartial))) != cudaSuccess ||
         (e = cudaMalloc((void**)&s->outlet_partials, sizeof(OutletCand) * s->reduce_blocks)) != cudaSuccess ||
         (e = cudaMalloc((void**)&s->d_outlet, sizeof(OutletCand))) != cudaSuccess ||
@@ -971,11 +1064,12 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
     if ((e = cudaMemsetAsync(s->w[0], 0, grid_bytes, s->stream)) != cudaSuccess ||
         (e = cudaMemsetAsync(s->w[1], 0, grid_bytes, s->stream)) != cudaSuccess ||
         (e = cudaMemsetAsync(s->oldw, 0, grid_bytes, s->stream)) != cudaSuccess ||
-        (e = cudaMemsetAsync(s->totaldrain, 0, 8 * kMaxOutlets, s->stream)) != cudaSuccess ||
-        (e = cudaMemsetAsync(s->flags, 0, sizeof(HaloFlags), s->stream)) != cudaSuccess ||
-        (e = cudaMemsetAsync(s->events, 0, ev_bytes, s->stream)) != cudaSuccess)
+        (e = cudaMemsetAsync(s->d_cta_outlets, 0, (size_t)s->n_strips * s->n_chunks, s->stream)) != cudaSuccess ||
+        (e = cudaMemsetAsync(s->flags, 0, kFlagsBytes + ev_bytes, s->stream)) != cudaSuccess)
         return cleanup(WDPM_E_CUDA, cudaGetErrorString(e));
-    int rc = s->dtype == WDPM_F64 ? fill_dem<double>(s) : fill_dem<float>(s);
+    int rc = alloc_outlets(s, 1);  // the single total exists before any set is installed
+    if (rc) { wdpm_destroy(s); return rc; }
+    rc = s->dtype == WDPM_F64 ? fill_dem<double>(s) : fill_dem<float>(s);
     if (rc) { wdpm_destroy(s); return rc; }
     if ((e = cudaStreamSynchronize(s->stream)) != cudaSuccess) return cleanup(WDPM_E_CUDA, cudaGetErrorString(e));
     *out = s;
@@ -993,7 +1087,8 @@ int wdpm_destroy(wdpm_solver* s) {
             cudaIpcCloseMemHandle(peer->flags);
         }
     if (s->flags) cudaFree(s->flags);
-    void* ptrs[] = {s->dem, s->w[0], s->w[1], s->oldw, s->totaldrain, s->saved_elev, s->d_outlet_rc, s->partials, s->d_result, s->outlet_partials, s->d_outlet, s->d_dirty};
+    void* ptrs[] = {s->dem, s->w[0], s->w[1], s->oldw, s->totaldrain, s->ev_area, s->saved_elev, s->d_outlet_rc, s->d_outlet_pos, s->d_cta_outlets,
+                    s->d_total, s->d_bad, s->partials, s->d_result, s->outlet_partials, s->d_outlet, s->d_dirty};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (s->h_result) cudaFreeHost(s->h_result);
@@ -1148,24 +1243,35 @@ int wdpm_set_outlets(wdpm_solver* s, int32_t n, const int32_t* rows, const int32
     if (n < 1 || n > kMaxOutlets) return fail(WDPM_E_ARG, "number of outlets must be in 1..WDPM_MAX_OUTLETS");
     if (n > 1 && s->schedule == WDPM_SCHEDULE_SERIAL) return fail(WDPM_E_UNSUPPORTED, "the serial schedule has one outlet (the emptying of overlapping outlet neighbourhoods is not defined)");
     if (s->in_block) return fail(WDPM_E_STATE, "a block is open");
-    for (int k = 0; k < n; k++) {
-        if (rows[k] < 0 || rows[k] > s->cfg.rows + 1 || cols[k] < 0 || cols[k] > s->g.C + 1) return fail(WDPM_E_ARG, "outlet outside the padded grid");
-        for (int q = 0; q < k; q++)
-            if (rows[q] == rows[k] && cols[q] == cols[k]) return fail(WDPM_E_ARG, "duplicate outlet");
-    }
+    for (int k = 0; k < n; k++)
+        if (rows[k] < 1 || rows[k] > s->cfg.rows || cols[k] < 1 || cols[k] > s->g.C) return fail(WDPM_E_ARG, "outlet outside the DEM");
+    // sort by (row, col): kernels find an outlet by binary search; order[i] = the caller's index of sorted outlet i
+    std::vector<int> order((size_t)n);
+    for (int k = 0; k < n; k++) order[k] = k;
+    auto key = [&](int k) { return ((long long)rows[k] << 32) | (long long)cols[k]; };
+    std::sort(order.begin(), order.end(), [&](int a, int b) { return key(a) < key(b); });
+    for (int i = 1; i < n; i++)
+        if (key(order[i]) == key(order[i - 1])) return fail(WDPM_E_ARG, "duplicate outlet");
     CUDA_TRY(cudaSetDevice(s->device));
     int rc = apply_outlet_marks(s, false);  // restore the cells of the previous set
     if (rc) return rc;
+    rc = alloc_outlets(s, n);
+    if (rc) { s->n_outlets = 0; s->have_outlet = false; return rc; }
     s->outlet_rc.resize((size_t)2 * n);
-    for (int k = 0; k < n; k++) {
-        s->outlet_rc[2 * k] = rows[k] - s->G;  // kernels work in the stripe's local rows (may lie outside the stripe)
-        s->outlet_rc[2 * k + 1] = cols[k];
+    s->outlet_pos.resize((size_t)n);
+    for (int i = 0; i < n; i++) {
+        s->outlet_rc[2 * i] = rows[order[i]] - s->G;  // kernels work in the stripe's local rows (may lie outside the stripe)
+        s->outlet_rc[2 * i + 1] = cols[order[i]];
+        s->outlet_pos[order[i]] = i;
     }
     s->n_outlets = n;
     s->have_outlet = true;
     CUDA_TRY(cudaMemcpyAsync(s->d_outlet_rc, s->outlet_rc.data(), sizeof(int) * 2 * n, cudaMemcpyHostToDevice, s->stream));
-    CUDA_TRY(cudaMemsetAsync(s->events, 0, (size_t)kEventSlots * n * kEventsPerBuffer * (s->dtype == WDPM_F64 ? sizeof(DrainEvent<double>) : sizeof(DrainEvent<float>)), s->stream));
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    CUDA_TRY(cudaMemcpyAsync(s->d_outlet_pos, s->outlet_pos.data(), sizeof(int) * n, cudaMemcpyHostToDevice, s->stream));
+    CUDA_TRY(cudaMemsetAsync(s->ev_area, 0, event_area_bytes(n, s->ev_slots, s->esize), s->stream));
+    if (s->events) CUDA_TRY(cudaMemsetAsync(s->events, 0, event_area_bytes(border_entries(s), s->ev_slots, s->esize), s->stream));
+    rc = s->dtype == WDPM_F64 ? compute_cta_outlets<double>(s) : compute_cta_outlets<float>(s);
+    if (rc) return rc;
     return s->have_dem ? apply_outlet_marks(s, true) : WDPM_OK;
 }
 
@@ -1174,39 +1280,54 @@ int wdpm_set_total_drain(wdpm_solver* s, double value) {
     CUDA_TRY(cudaSetDevice(s->device));
     double v64 = value;
     float v32 = (float)value;
-    CUDA_TRY(cudaMemsetAsync(s->totaldrain, 0, 8 * kMaxOutlets, s->stream));  // the value goes to the first outlet's total
-    CUDA_TRY(cudaMemcpyAsync(s->totaldrain, s->dtype == WDPM_F64 ? (void*)&v64 : (void*)&v32, s->esize, cudaMemcpyHostToDevice, s->stream));
+    const size_t first = s->n_outlets > 0 ? (size_t)s->outlet_pos[0] : 0;  // the value goes to the first outlet's total
+    CUDA_TRY(cudaMemsetAsync(s->totaldrain, 0, s->esize * s->outlet_cap, s->stream));
+    CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(s->totaldrain) + first * s->esize, s->dtype == WDPM_F64 ? (void*)&v64 : (void*)&v32, s->esize,
+                             cudaMemcpyHostToDevice, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    return WDPM_OK;
+}
+
+int wdpm_seed_outlet_drains(wdpm_solver* s) {
+    if (!s) return fail(WDPM_E_ARG, "null solver");
+    if (!s->have_dem) return fail(WDPM_E_STATE, "upload first");
+    if (!s->have_outlet) return fail(WDPM_E_STATE, "no outlet installed");
+    if (s->in_block) return fail(WDPM_E_STATE, "a block is open");
+    CUDA_TRY(cudaSetDevice(s->device));
+    const int blocks = (s->n_outlets + 255) / 256;
+    if (s->dtype == WDPM_F64) k_seed_outlets<double><<<blocks, 256, 0, s->stream>>>(static_cast<const double*>(s->w[s->cur]), s->g, drain_state<double>(s));
+    else k_seed_outlets<float><<<blocks, 256, 0, s->stream>>>(static_cast<const float*>(s->w[s->cur]), s->g, drain_state<float>(s));
+    s->launches++;
+    CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaStreamSynchronize(s->stream));
     return WDPM_OK;
 }
 
 int wdpm_get_outlet_drains(wdpm_solver* s, double* values, int32_t n) {
     if (!s || !values) return fail(WDPM_E_ARG, "null argument");
-    if (n < 1 || n > kMaxOutlets) return fail(WDPM_E_ARG, "n out of range");
+    if (n < 1 || n > s->outlet_cap) return fail(WDPM_E_ARG, "n out of range (at most the installed set's size)");
     CUDA_TRY(cudaSetDevice(s->device));
-    std::vector<double> v64((size_t)n);
-    std::vector<float> v32((size_t)n);
-    CUDA_TRY(cudaMemcpyAsync(s->dtype == WDPM_F64 ? (void*)v64.data() : (void*)v32.data(), s->totaldrain, s->esize * (size_t)n, cudaMemcpyDeviceToHost, s->stream));
+    const size_t m = (size_t)s->outlet_cap;
+    std::vector<double> v64(s->dtype == WDPM_F64 ? m : 0);
+    std::vector<float> v32(s->dtype == WDPM_F64 ? 0 : m);
+    CUDA_TRY(cudaMemcpyAsync(s->dtype == WDPM_F64 ? (void*)v64.data() : (void*)v32.data(), s->totaldrain, s->esize * m, cudaMemcpyDeviceToHost, s->stream));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
-    for (int k = 0; k < n; k++) values[k] = s->dtype == WDPM_F64 ? v64[k] : (double)v32[k];
+    for (int k = 0; k < n; k++) {  // back to the caller's order
+        const size_t i = s->n_outlets > 0 ? (size_t)s->outlet_pos[k] : (size_t)k;
+        values[k] = s->dtype == WDPM_F64 ? v64[i] : (double)v32[i];
+    }
     return WDPM_OK;
 }
 
 int wdpm_get_total_drain(wdpm_solver* s, double* value) {
     if (!s || !value) return fail(WDPM_E_ARG, "null argument");
-    const int n = s->n_outlets > 0 ? s->n_outlets : 1;
-    std::vector<double> v((size_t)n);
-    int rc = wdpm_get_outlet_drains(s, v.data(), n);
-    if (rc) return rc;
-    if (s->dtype == WDPM_F64) {
-        double t = v[0];
-        for (int k = 1; k < n; k++) t = t + v[k];
-        *value = t;
-    } else {
-        float t = (float)v[0];
-        for (int k = 1; k < n; k++) t = t + (float)v[k];
-        *value = (double)t;
-    }
+    CUDA_TRY(cudaSetDevice(s->device));
+    if (s->dtype == WDPM_F64) k_sum_totals<double><<<1, 32, 0, s->stream>>>(static_cast<const double*>(s->totaldrain), s->d_outlet_pos, std::max(s->n_outlets, 1), s->d_total);
+    else k_sum_totals<float><<<1, 32, 0, s->stream>>>(static_cast<const float*>(s->totaldrain), s->d_outlet_pos, std::max(s->n_outlets, 1), s->d_total);
+    s->launches++;
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(value, s->d_total, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
     return WDPM_OK;
 }
 
@@ -1468,7 +1589,8 @@ int wdpm_stripe_upload(wdpm_solver* s, const void* dem_band, const void* water_b
     CUDA_TRY(cudaMemsetAsync(s->flags, 0, sizeof(HaloFlags), s->stream));
     s->epoch = 0;
     s->launch_slot = 0;  // neighbours must agree on the event buffer rotation as well
-    CUDA_TRY(cudaMemsetAsync(s->events, 0, (size_t)kEventSlots * kMaxOutlets * kEventsPerBuffer * (s->dtype == WDPM_F64 ? sizeof(DrainEvent<double>) : sizeof(DrainEvent<float>)), s->stream));
+    CUDA_TRY(cudaMemsetAsync(s->ev_area, 0, event_area_bytes(s->outlet_cap, s->ev_slots, s->esize), s->stream));
+    if (s->events) CUDA_TRY(cudaMemsetAsync(s->events, 0, event_area_bytes(border_entries(s), s->ev_slots, s->esize), s->stream));
     s->halo_failed = false;
     *s->h_halo_error = 0;
     s->have_dem = true;

@@ -30,6 +30,19 @@
  * (0 auto, 1 colour, 2 fused, 3 resident), WDPM_B200_GPUS (number of GPUs, default 1:
  * the DEM is cut into that many row stripes, one solver per GPU, halos exchanged over
  * NVLink by the library; results do not depend on the count).
+ *
+ * Extension, Drain modules only (chained ones too): WDPM_B200_OUTLETS replaces the reference's single outlet
+ * (the lowest cell with dem > 0) by a set of outlets, each with its own drained total (wdpm_set_outlets):
+ *   WDPM_B200_OUTLETS=rim     every cell with dem > nodata in the first or last row or column of the DEM;
+ *   WDPM_B200_OUTLETS=<path>  an ESRI ASCII grid of the DEM's ncols and nrows: every cell whose value is > 0
+ *                             and not the grid's NODATA value is an outlet.
+ * Outlets are taken in row-major order. Fewer than one, more than WDPM_MAX_OUTLETS, an outlet on a cell with
+ * dem <= nodata, a grid of another size, or a set of more than one outlet with cpu=0 (the serial branch drains
+ * one outlet) print a message and exit with 1. Each total starts at max(water at its outlet, 0)
+ * (wdpm_seed_outlet_drains, WDPMCL.c:1029 per outlet). The report prints "Drain outlets:" and the lowest
+ * outlet elevation instead of the drain column, row and elevation; "Volume drained" is the sum of the totals
+ * in outlet order. WDPM_B200_OUTLET_TOTALS=<path> also writes one CSV line per outlet at the end, in outlet
+ * order: row,col,elevation_m,drained_m3 (1-based padded coordinates, values as %.17g).
  */
 #define _POSIX_C_SOURCE 200809L
 #include <ctype.h>
@@ -403,6 +416,62 @@ static int write_grid(const char *path, const asc_header *h, const double *g)
     return failed ? -1 : 0;
 }
 
+/* ---- drain outlet sets (WDPM_B200_OUTLETS) ------------------------------------ */
+
+typedef struct {
+    int32_t n;
+    int32_t *row, *col; /* 1-based padded coordinates, row-major order */
+} outlet_set;
+
+static void outlets_fail(const char *spec, const char *why)
+{
+    fprintf(stderr, "Couldn't use the drain outlets WDPM_B200_OUTLETS=%s: %s\n", spec, why);
+    exit(1);
+}
+
+/* The set WDPM_B200_OUTLETS names, checked against the DEM before any solver exists. */
+static void load_outlets(const char *spec, const double *dem, int rows, int cols, double nodata, outlet_set *os)
+{
+    const size_t n = (size_t)rows * (size_t)cols;
+    unsigned char *is_out = calloc(n, 1);
+    if (!is_out) outlets_fail(spec, "out of memory");
+    if (!strcmp(spec, "rim")) {
+        for (int i = 0; i < rows; i++)
+            for (int j = 0; j < cols; j++)
+                if (i == 0 || i == rows - 1 || j == 0 || j == cols - 1) is_out[(size_t)i * cols + j] = dem[(size_t)i * cols + j] > nodata;
+    } else {
+        char *hb = slurp(spec, NULL);
+        asc_header h;
+        if (!hb || !parse_header(hb, &h)) outlets_fail(spec, "not a readable ESRI ASCII grid");
+        free(hb);
+        if (h.ncols != cols || h.nrows != rows) outlets_fail(spec, "its ncols and nrows differ from the DEM's");
+        double *g = read_grid(spec, rows, cols, 0.0, NULL);
+        if (!g) outlets_fail(spec, "not a readable ESRI ASCII grid");
+        for (size_t k = 0; k < n; k++) is_out[k] = g[k] > 0 && g[k] != h.nodata;
+        free(g);
+    }
+    size_t cnt = 0;
+    for (size_t k = 0; k < n; k++) {
+        if (!is_out[k]) continue;
+        if (!(dem[k] > nodata)) outlets_fail(spec, "an outlet lies on a cell with dem <= nodata");
+        cnt++;
+    }
+    if (cnt == 0) outlets_fail(spec, "no outlet");
+    if (cnt > WDPM_MAX_OUTLETS) outlets_fail(spec, "more outlets than WDPM_MAX_OUTLETS");
+    os->n = (int32_t)cnt;
+    os->row = malloc(cnt * sizeof *os->row);
+    os->col = malloc(cnt * sizeof *os->col);
+    if (!os->row || !os->col) outlets_fail(spec, "out of memory");
+    cnt = 0;
+    for (size_t k = 0; k < n; k++)
+        if (is_out[k]) {
+            os->row[cnt] = (int32_t)(k / (size_t)cols) + 1;
+            os->col[cnt] = (int32_t)(k % (size_t)cols) + 1;
+            cnt++;
+        }
+    free(is_out);
+}
+
 /* ---- run ------------------------------------------------------------------- */
 
 static double seconds_since(const struct timeval *t0)
@@ -569,6 +638,23 @@ typedef struct {
 } chain_state;
 
 static int run_module(int ntok, char tok[][512], int argc, chain_state *cs);
+
+/* Every outlet's total over the stripes (each total lives on the stripe that owns the outlet's row and reads 0
+ * elsewhere, so the element-wise sum is exact) and their sum in outlet order, the single-GPU block total. */
+static double set_outlet_totals(solver_set *ss, const outlet_set *os, double *totals)
+{
+    double *part = ss->n > 1 ? malloc((size_t)os->n * sizeof *part) : NULL;
+    if (ss->n > 1 && !part) die_solver("allocate outlet totals");
+    for (int g = 0; g < ss->n; g++) {
+        if (wdpm_get_outlet_drains(ss->sv[g], g == 0 ? totals : part, os->n) != WDPM_OK) die_solver("read outlet totals");
+        if (g > 0)
+            for (int32_t k = 0; k < os->n; k++) totals[k] += part[k];
+    }
+    free(part);
+    double t = totals[0];
+    for (int32_t k = 1; k < os->n; k++) t = t + totals[k];
+    return t;
+}
 
 int main(int argc, char **argv)
 {
@@ -740,6 +826,16 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         initial_vol *= cellarea;
     }
 
+    /* an outlet set replaces the reference's single outlet (Drain only); checked before any solver exists */
+    outlet_set os = {0, NULL, NULL};
+    const char *outlet_spec = getenv("WDPM_B200_OUTLETS");
+    if (is_drain && outlet_spec && *outlet_spec) {
+        load_outlets(outlet_spec, dem, rows, cols, nodata, &os);
+        if (a.backend == 0 && os.n > 1) outlets_fail(outlet_spec, "cpu=0 (the serial branch) drains through one outlet");
+    }
+    double *outlet_totals = os.n > 0 ? malloc((size_t)os.n * sizeof *outlet_totals) : NULL;
+    if (os.n > 0 && !outlet_totals) outlets_fail(outlet_spec, "out of memory");
+
     /* solver */
     wdpm_config cfg;
     memset(&cfg, 0, sizeof cfg);
@@ -778,7 +874,24 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     }
 
     double total_drain = 0.0;
-    if (is_drain) {
+    if (is_drain && os.n > 0) {
+        double minel = 0.0;
+        for (int32_t k = 0; k < os.n; k++) {
+            const double e = dem[(size_t)(os.row[k] - 1) * cols + (os.col[k] - 1)];
+            if (k == 0 || e < minel) minel = e;
+        }
+        for (int g = 0; g < ss.n; g++) {
+            if (wdpm_set_outlets(ss.sv[g], os.n, os.row, os.col) != WDPM_OK) die_solver("set the drain outlets");
+            if (wdpm_seed_outlet_drains(ss.sv[g]) != WDPM_OK) die_solver("seed the outlet totals");
+        }
+        total_drain = set_outlet_totals(&ss, &os, outlet_totals);
+        line("               ");
+        printf("%30s\n", "Basin summary");
+        printf("%20s %10.4f %s\n", "Basin area:", (double)basincount * cellarea, "m2");
+        printf("%20s %10.4f %s\n", "Initial volume:", initial_vol, "m3");
+        printf("%20s %d\n", "Drain outlets:", os.n);
+        printf("%20s %10.4f %s\n", "Min DEM elevation:", minel, "m");
+    } else if (is_drain) {
         int32_t drow = 0, dcol = 0;
         double minel = 0.0, w_out = 0.0;
         int owner = -1;
@@ -824,7 +937,7 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         wdpm_block_result r;
         set_run_block(&ss, BLOCK_ITERATIONS, &r);
         k += BLOCK_ITERATIONS;
-        total_drain = r.total_drain;
+        total_drain = (os.n > 0 && ss.n > 1) ? set_outlet_totals(&ss, &os, outlet_totals) : r.total_drain;
         double diffdrain = 0.0;
         if (is_drain) {
             diffdrain = fabs(total_drain - old_drain) * cellarea;
@@ -900,6 +1013,24 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         return 1;
     }
     printf("%20s %10.2f %s\n", "Run Time", seconds_since(&t0), "s");
+    const char *totals_path = getenv("WDPM_B200_OUTLET_TOTALS");
+    if (os.n > 0 && totals_path && *totals_path) {
+        set_outlet_totals(&ss, &os, outlet_totals);
+        FILE *f = fopen(totals_path, "w");
+        if (!f) {
+            perror("Couldn't write the outlet totals");
+            return 1;
+        }
+        for (int32_t q = 0; q < os.n; q++)
+            fprintf(f, "%d,%d,%.17g,%.17g\n", os.row[q], os.col[q], dem[(size_t)(os.row[q] - 1) * cols + (os.col[q] - 1)], outlet_totals[q] * cellarea);
+        if (fclose(f) != 0) {
+            perror("Couldn't write the outlet totals");
+            return 1;
+        }
+    }
+    free(outlet_totals);
+    free(os.row);
+    free(os.col);
     free(scratch.grid);
     if (cs) { /* keep what the next module may want: the solver (grids in HBM) and the output as its file reads back */
         cs->prev = ss;

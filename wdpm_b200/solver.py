@@ -18,6 +18,7 @@ F32, F64 = 0, 1
 KERNEL_AUTO, KERNEL_COLOUR, KERNEL_FUSED, KERNEL_RESIDENT = 0, 1, 2, 3
 # update schedule (WDPM_SCHEDULE_* in include/wdpm_b200.h): the reference's OpenCL branch, or its serial branch
 SCHED_OPENCL, SCHED_SERIAL = 0, 1
+MAX_OUTLETS = 1 << 20  # WDPM_MAX_OUTLETS: the largest outlet set wdpm_set_outlets takes
 MODULES = {"add": ADD, "subtract": SUBTRACT, "drain": DRAIN}
 # the tiling AUTO picks for large fp64 Add/Subtract grids (kDefaultVariantF64 in csrc/solver.cu); tests and
 # smoke() name it to exercise the production kernel on small grids
@@ -199,6 +200,11 @@ class Solver:
         cols = (C.c_int32 * len(outlets))(*[int(o[1]) for o in outlets])
         _check(self._lib.wdpm_set_outlets(self._h, C.c_int32(len(outlets)), rows, cols))
         self.n_outlets = len(outlets)
+
+    def seed_outlet_drains(self):
+        """Every outlet's total = max(water at the outlet, 0) (WDPMCL.c:1029 per outlet); on row stripes only the
+        stripe that owns the outlet's row keeps a non-zero seed."""
+        _check(self._lib.wdpm_seed_outlet_drains(self._h))
 
     def get_outlet_drains(self, n: int) -> np.ndarray:
         out = np.zeros(n, dtype=np.float64)

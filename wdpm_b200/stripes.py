@@ -151,6 +151,13 @@ class DistributedSolver:
             out.total_drain = float(acc)
         return out
 
+    def set_outlets(self, outlets):
+        """Every stripe takes the whole set (padded (row, col) of the whole DEM)."""
+        self.solver.set_outlets(outlets)
+
+    def seed_outlet_drains(self):
+        self.solver.seed_outlet_drains()
+
     def outlet_drains(self, n: int) -> np.ndarray:
         """Per-outlet totals of the whole DEM: each is kept by the stripe that owns the outlet's row (0 elsewhere),
         so the element-wise sum over the stripes is exact."""

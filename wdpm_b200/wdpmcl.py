@@ -53,10 +53,11 @@ class RunReport:
     mean_water: float
     drain_depth: float
     max_depth_mm: float
-    outlet: tuple | None
-    min_elevation: float | None
+    outlet: tuple | None        # the reference's single outlet (None when a set was given)
+    min_elevation: float | None  # its elevation, or the lowest outlet elevation of a set
     solver_ms: float
     launches: int
+    outlet_totals: np.ndarray | None = None  # a set: every outlet's drained depth in m (x cellarea = m3), in outlet order
 
 
 def default_backend(dtype=_solver.F64, **kw) -> Callable:
@@ -66,12 +67,15 @@ def default_backend(dtype=_solver.F64, **kw) -> Callable:
 
 
 def run_module(dem: np.ndarray, nodata: float, cellsize: float, params: ModuleParams, water: np.ndarray | None = None,
-               backend: Callable | None = None, resume: bool = False, on_block: Callable | None = None) -> RunReport:
+               backend: Callable | None = None, resume: bool = False, on_block: Callable | None = None,
+               outlets=None) -> RunReport:
     """Run one module to its stop criterion.
 
     `water` is the water-file contents (None = "NULL"/absent). `resume=True` means
     `water` came from a scratch file: the module's add/subtract step is skipped
-    (WDPMCL.c:668-673, :824-829).
+    (WDPMCL.c:668-673, :824-829). `outlets` (Drain only): None for the reference's
+    single outlet, a list of 1-based (row, col), or "rim" (ascgrid.rim_outlets) -
+    the water then leaves through every outlet of the set, each with its own total.
     """
     import time
 
@@ -110,7 +114,15 @@ def run_module(dem: np.ndarray, nodata: float, cellsize: float, params: ModulePa
 
     outlet = None
     min_elev = None
-    if params.module == "drain":
+    if outlets is not None and params.module == "drain":
+        from .ascgrid import rim_outlets
+        outlets = rim_outlets(dem, nodata) if isinstance(outlets, str) and outlets == "rim" else [(int(r), int(c)) for r, c in outlets]
+        if not outlets:
+            raise ValueError("the outlet set is empty")
+        be.set_outlets(outlets)
+        be.seed_outlet_drains()
+        min_elev = min(float(dem[r - 1, c - 1]) for r, c in outlets)
+    elif params.module == "drain":
         r, c, min_elev = be.find_outlet()
         outlet = (r, c)
         w_out = be.get_cell_water(r, c)
@@ -146,6 +158,7 @@ def run_module(dem: np.ndarray, nodata: float, cellsize: float, params: ModulePa
             break
 
     w = be.download_water().astype(np.float64)
+    outlet_totals = be.get_outlet_drains(len(outlets)) if outlets is not None and params.module == "drain" else None
     if hasattr(be, "close"):
         be.close()
 
@@ -162,4 +175,4 @@ def run_module(dem: np.ndarray, nodata: float, cellsize: float, params: ModulePa
     drain_depth = (drain_vol / (float(np.float32(basincount)) * cellarea)) * 1000 if params.module == "drain" else 0.0
     max_depth_mm = float(np.max(w)) * 1000  # scans every cell, NODATA included (WDPMCL.c:1451-1459)
     return RunReport(w, k, blocks, initial_vol, final_vol, drain_vol, water_frac, mean_water, drain_depth, max_depth_mm,
-                     outlet, min_elev, solver_ms, launches)
+                     outlet, min_elev, solver_ms, launches, outlet_totals)
