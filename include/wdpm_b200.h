@@ -165,6 +165,26 @@ int wdpm_get_total_drain(wdpm_solver *s, double *value);
  * stripes the stripe that owns the outlet's row does it and the others set 0. For one outlet it equals
  * wdpm_get_cell_water followed by wdpm_set_total_drain(max(w, 0)). */
 int wdpm_seed_outlet_drains(wdpm_solver *s);
+/* Restore every outlet's total, values[k] for the caller's outlet k (n = the installed set's size; 1 for the
+ * reference's outlet or before any set). On row stripes it follows wdpm_seed_outlet_drains: the stripe that owns the
+ * outlet's row keeps the value and the others set 0, so every stripe may be given the whole array. Converted to the
+ * solver's precision. WDPM_E_STATE outside Drain, WDPM_E_ARG for another n. Resumes a Drain run with its totals
+ * (wdpm_set_total_drain keeps only the first outlet's). */
+int wdpm_set_outlet_drains(wdpm_solver *s, const double *values, int32_t n);
+/* Exact checkpoints. wdpm_checkpoint_arm makes the next wdpm_block_begin (or wdpm_run_block) capture the state the
+ * block starts from: the water after its zero-threshold pass (the snapshot of src/WDPMCL.c:1055-1073; the pass is
+ * idempotent, so this water starts a block exactly as the unthresholded water before it does) and every outlet's
+ * total. The block runs on while a side stream copies both into pinned host memory the solver owns (allocated by
+ * the first arm, one owned grid, freed by wdpm_destroy); nothing waits for the copy on the host, and the next
+ * prologue waits for it on the device. wdpm_checkpoint_wait blocks until the capture has landed and returns
+ * pointers into that memory, valid until the next arm: the water as the owned interior rows (unpadded row-major, the
+ * solver's precision, raw bits; a stripe's rows as wdpm_download_water returns them) and the totals as doubles in
+ * the caller's outlet order (n = the set's size, 1 without a set; per stripe as wdpm_get_outlet_drains). Uploading
+ * that water into a fresh solver for the same DEM and module (any kernel, any partition) and restoring the totals
+ * with wdpm_set_outlet_drains continues the run bit for bit. arm: WDPM_E_STATE inside a block or before an
+ * upload; wait: WDPM_E_STATE when no capture has been taken since the last arm. */
+int wdpm_checkpoint_arm(wdpm_solver *s);
+int wdpm_checkpoint_wait(wdpm_solver *s, const void **water, const double **totals, int32_t *n);
 /* Module chaining. The reference runs Add -> Drain -> Subtract as three processes that hand the
  * water grid on through "%f" text files (validation/validate_WDPM.sh:77-99). A host that runs the
  * modules in one process can keep the grids in HBM instead:

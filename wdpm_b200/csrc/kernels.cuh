@@ -489,6 +489,12 @@ __global__ void k_sum_totals(const T* __restrict__ totals, const int* __restrict
     *out = (double)t;
 }
 
+// Checkpoint capture: the outlets' totals in the caller's order, widened to double (exact for both precisions).
+template <typename T>
+__global__ void k_gather_totals(const T* __restrict__ totals, const int* __restrict__ pos, int n, double* __restrict__ out) {
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) out[k] = (double)totals[pos[k]];
+}
+
 // Record one event: its addends go into slot `slot` of `entry` in buffer `buffer` of area `a`. `sys`: a border
 // area, into which the neighbour's centres record from another GPU too (system-scope atomics); only this solver's
 // kernels write its outlet area.

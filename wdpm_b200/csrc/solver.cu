@@ -316,6 +316,18 @@ struct wdpm_solver {
     bool in_block = false;
     long long blk_launches0 = 0;
     int blk_iters = 0;
+
+    // Checkpoint capture (wdpm_checkpoint_arm / wdpm_checkpoint_wait): an armed block prologue gathers the totals,
+    // and a side stream copies the snapshot it wrote (oldw) and those totals into pinned staging while the block
+    // runs. ck_done marks the copies' completion; every later writer of oldw or d_ck_totals waits on it on the
+    // device (ck_fence).
+    cudaStream_t ck_stream = nullptr;
+    cudaEvent_t ck_ready = nullptr, ck_done = nullptr;
+    bool ck_armed = false, ck_captured = false;
+    void* ck_water = nullptr;       // pinned: the owned interior rows, unpadded, solver precision
+    double* ck_totals = nullptr;    // pinned: ck_cap totals
+    double* d_ck_totals = nullptr;  // device: ck_cap totals, the gather's output
+    int ck_cap = 0, ck_n = 0;
 };
 
 namespace {
@@ -618,6 +630,56 @@ int iterate(wdpm_solver* s, int n) {
     return s->dtype == WDPM_F64 ? iterate_t<double>(s, n) : iterate_t<float>(s, n);
 }
 
+// The interior rows this solver owns in a device grid: address of the first one's first cell, and their number
+// (all rows of a single solver; a stripe's owned rows clipped to the DEM).
+const char* owned_interior(const wdpm_solver* s, const void* base, int* n_rows) {
+    const int lo = std::max(s->G, 1), hi = std::min(s->G + s->P, s->cfg.rows + 1);
+    *n_rows = hi - lo;
+    return static_cast<const char*>(base) + ((size_t)(lo - s->G + kPadTop) * s->g.pitch + (size_t)(1 + kPadLeft)) * s->esize;
+}
+
+// Device-side ordering against the last checkpoint capture: work enqueued after this on the solver stream starts
+// only once the capture's copies out of oldw and d_ck_totals have completed.
+int ck_fence(wdpm_solver* s) {
+    if (s->ck_done) CUDA_TRY(cudaStreamWaitEvent(s->stream, s->ck_done, 0));
+    return WDPM_OK;
+}
+
+// An armed capture, right after the prologue: gather the totals, then copy them and the snapshot to the staging on
+// the side stream, which waits for the prologue and the gather on the device.
+template <typename T>
+int capture_t(wdpm_solver* s) {
+    // sized here, not at the arm: a larger outlet set may have been installed since
+    const int n = std::max(s->n_outlets, 1);
+    if (n > s->ck_cap) {
+        CUDA_TRY(cudaStreamSynchronize(s->ck_stream));  // the last capture's copy still reads the old arrays
+        if (s->ck_totals) cudaFreeHost(s->ck_totals);
+        if (s->d_ck_totals) cudaFree(s->d_ck_totals);
+        s->ck_totals = s->d_ck_totals = nullptr;
+        s->device_bytes -= (long long)sizeof(double) * s->ck_cap;
+        s->ck_cap = 0;
+        CUDA_TRY(cudaHostAlloc((void**)&s->ck_totals, sizeof(double) * n, cudaHostAllocDefault));
+        CUDA_TRY(cudaMalloc((void**)&s->d_ck_totals, sizeof(double) * n));
+        s->ck_cap = n;
+        s->device_bytes += (long long)sizeof(double) * n;
+    }
+    k_gather_totals<T><<<(n + 255) / 256, 256, 0, s->stream>>>(static_cast<const T*>(s->totaldrain), s->d_outlet_pos, n, s->d_ck_totals);
+    s->launches++;
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(s->ck_ready, s->stream));
+    CUDA_TRY(cudaStreamWaitEvent(s->ck_stream, s->ck_ready, 0));
+    int rows = 0;
+    const char* src = owned_interior(s, s->oldw, &rows);
+    CUDA_TRY(cudaMemcpy2DAsync(s->ck_water, (size_t)s->g.C * s->esize, src, (size_t)s->g.pitch * s->esize, (size_t)s->g.C * s->esize,
+                               (size_t)rows, cudaMemcpyDeviceToHost, s->ck_stream));
+    CUDA_TRY(cudaMemcpyAsync(s->ck_totals, s->d_ck_totals, sizeof(double) * n, cudaMemcpyDeviceToHost, s->ck_stream));
+    CUDA_TRY(cudaEventRecord(s->ck_done, s->ck_stream));
+    s->ck_armed = false;
+    s->ck_captured = true;
+    s->ck_n = n;
+    return WDPM_OK;
+}
+
 // A block in three non-blocking-then-blocking pieces (see wdpm_block_begin/enqueue/end).
 template <typename T>
 int block_begin_t(wdpm_solver* s) {
@@ -625,6 +687,10 @@ int block_begin_t(wdpm_solver* s) {
     s->blk_launches0 = s->launches;
     s->blk_iters = 0;
     CUDA_TRY(cudaEventRecord(s->ev[0], s->stream));
+    {   // the prologue overwrites oldw, and an armed one the gathered totals: not before the last capture is out
+        const int rc = ck_fence(s);
+        if (rc) return rc;
+    }
     if (s->stripe && s->epoch > 0 && (s->above.present || s->below.present)) {
         // the neighbours' last halo push must land before the threshold pass touches the halo rows
         k_halo_wait<<<1, 32, 0, s->stream>>>(s->flags, s->above.present, s->below.present, s->epoch, s->halo_timeout_ns);
@@ -637,6 +703,10 @@ int block_begin_t(wdpm_solver* s) {
         static_cast<T*>(s->w[s->cur]), static_cast<T*>(s->oldw), static_cast<const T*>(s->dem), n, (T)s->cfg.zero_threshold, s->d_dirty);
     s->launches++;
     CUDA_TRY(cudaGetLastError());
+    if (s->ck_armed) {
+        const int rc = capture_t<T>(s);
+        if (rc) return rc;
+    }
     CUDA_TRY(cudaEventRecord(s->ev[1], s->stream));
     s->in_block = true;
     return WDPM_OK;
@@ -1080,6 +1150,13 @@ int wdpm_destroy(wdpm_solver* s) {
     if (!s) return WDPM_OK;
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
+    if (s->ck_done) cudaEventSynchronize(s->ck_done);  // a capture may still be copying out of oldw
+    if (s->ck_water) cudaFreeHost(s->ck_water);
+    if (s->ck_totals) cudaFreeHost(s->ck_totals);
+    if (s->d_ck_totals) cudaFree(s->d_ck_totals);
+    if (s->ck_ready) cudaEventDestroy(s->ck_ready);
+    if (s->ck_done) cudaEventDestroy(s->ck_done);
+    if (s->ck_stream) cudaStreamDestroy(s->ck_stream);
     for (auto* peer : {&s->above, &s->below})
         if (peer->present && peer->ipc) {
             cudaIpcCloseMemHandle(peer->w[0]);
@@ -1155,16 +1232,10 @@ int wdpm_download_water(wdpm_solver* s, void* water) {
     if (!s || !water) return fail(WDPM_E_ARG, "null argument");
     if (!s->have_dem) return fail(WDPM_E_STATE, "nothing uploaded yet");
     CUDA_TRY(cudaSetDevice(s->device));
-    if (s->stripe) {  // the owned interior rows only
-        const int lo = (s->G > 1 ? s->G : 1), hi = (s->G + s->P < s->cfg.rows + 1 ? s->G + s->P : s->cfg.rows + 1);
-        const char* src = static_cast<const char*>(s->w[s->cur]) + ((size_t)(lo - s->G + kPadTop) * s->g.pitch + (size_t)(1 + kPadLeft)) * s->esize;
-        CUDA_TRY(cudaMemcpy2DAsync(water, (size_t)s->g.C * s->esize, src, (size_t)s->g.pitch * s->esize, (size_t)s->g.C * s->esize,
-                                   (size_t)(hi - lo), cudaMemcpyDeviceToHost, s->stream));
-        CUDA_TRY(cudaStreamSynchronize(s->stream));
-        return WDPM_OK;
-    }
-    CUDA_TRY(cudaMemcpy2DAsync(water, (size_t)s->g.C * s->esize, interior_ptr(s, s->w[s->cur]), (size_t)s->g.pitch * s->esize,
-                               (size_t)s->g.C * s->esize, (size_t)s->g.R, cudaMemcpyDeviceToHost, s->stream));
+    int rows = 0;  // a stripe: the owned interior rows only
+    const char* src = owned_interior(s, s->w[s->cur], &rows);
+    CUDA_TRY(cudaMemcpy2DAsync(water, (size_t)s->g.C * s->esize, src, (size_t)s->g.pitch * s->esize, (size_t)s->g.C * s->esize,
+                               (size_t)rows, cudaMemcpyDeviceToHost, s->stream));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
     return WDPM_OK;
 }
@@ -1328,6 +1399,57 @@ int wdpm_get_total_drain(wdpm_solver* s, double* value) {
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(value, s->d_total, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
+    return WDPM_OK;
+}
+
+int wdpm_set_outlet_drains(wdpm_solver* s, const double* values, int32_t n) {
+    if (!s || !values) return fail(WDPM_E_ARG, "null argument");
+    if (s->module != WDPM_DRAIN) return fail(WDPM_E_STATE, "outlet totals belong to the Drain module");
+    if (s->in_block) return fail(WDPM_E_STATE, "a block is open");
+    if (n != std::max(s->n_outlets, 1)) return fail(WDPM_E_ARG, "n must be the installed outlet set's size");
+    CUDA_TRY(cudaSetDevice(s->device));
+    // sorted order; as wdpm_seed_outlet_drains: a total is kept by the solver that owns its outlet's row, 0 elsewhere
+    std::vector<double> v64(s->dtype == WDPM_F64 ? (size_t)s->outlet_cap : 0, 0.0);
+    std::vector<float> v32(s->dtype == WDPM_F64 ? 0 : (size_t)s->outlet_cap, 0.0f);
+    for (int k = 0; k < n; k++) {
+        const size_t i = s->n_outlets > 0 ? (size_t)s->outlet_pos[k] : 0;
+        const bool owned = s->n_outlets == 0 || (s->outlet_rc[2 * i] >= 0 && s->outlet_rc[2 * i] < s->P);
+        if (s->dtype == WDPM_F64) v64[i] = owned ? values[k] : 0.0;
+        else v32[i] = owned ? (float)values[k] : 0.0f;
+    }
+    CUDA_TRY(cudaMemcpyAsync(s->totaldrain, s->dtype == WDPM_F64 ? (const void*)v64.data() : (const void*)v32.data(), s->esize * s->outlet_cap,
+                             cudaMemcpyHostToDevice, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    return WDPM_OK;
+}
+
+int wdpm_checkpoint_arm(wdpm_solver* s) {
+    if (!s) return fail(WDPM_E_ARG, "null solver");
+    if (!s->have_dem) return fail(WDPM_E_STATE, "upload first");
+    if (s->in_block) return fail(WDPM_E_STATE, "a block is open: arm before wdpm_block_begin");
+    CUDA_TRY(cudaSetDevice(s->device));
+    if (!s->ck_stream) CUDA_TRY(cudaStreamCreateWithFlags(&s->ck_stream, cudaStreamNonBlocking));
+    if (!s->ck_ready) CUDA_TRY(cudaEventCreateWithFlags(&s->ck_ready, cudaEventDisableTiming));
+    if (!s->ck_done) CUDA_TRY(cudaEventCreateWithFlags(&s->ck_done, cudaEventDisableTiming));
+    if (!s->ck_water) {
+        int rows = 0;
+        owned_interior(s, s->oldw, &rows);
+        CUDA_TRY(cudaHostAlloc(&s->ck_water, (size_t)rows * s->g.C * s->esize, cudaHostAllocDefault));
+    }
+    s->ck_armed = true;
+    s->ck_captured = false;
+    return WDPM_OK;
+}
+
+int wdpm_checkpoint_wait(wdpm_solver* s, const void** water, const double** totals, int32_t* n) {
+    if (!s) return fail(WDPM_E_ARG, "null solver");
+    if (!s->ck_captured)
+        return fail(WDPM_E_STATE, s->ck_armed ? "the armed capture is taken by the next wdpm_block_begin" : "no checkpoint capture armed");
+    CUDA_TRY(cudaSetDevice(s->device));
+    CUDA_TRY(cudaEventSynchronize(s->ck_done));
+    if (water) *water = s->ck_water;
+    if (totals) *totals = s->ck_totals;
+    if (n) *n = s->ck_n;
     return WDPM_OK;
 }
 

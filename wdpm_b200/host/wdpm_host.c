@@ -43,16 +43,29 @@
  * outlet elevation instead of the drain column, row and elevation; "Volume drained" is the sum of the totals
  * in outlet order. WDPM_B200_OUTLET_TOTALS=<path> also writes one CSV line per outlet at the end, in outlet
  * order: row,col,elevation_m,drained_m3 (1-based padded coordinates, values as %.17g).
+ *
+ * Extension, not under chain: exact checkpoints (wdpm_checkpoint_arm / wdpm_checkpoint_wait; file format at
+ * ck_header). WDPM_B200_CHECKPOINT=<path> writes one every WDPM_B200_CHECKPOINT_EVERY blocks (default 1) and one at
+ * the end; a "%d" in the path becomes the iteration count. Mid-run ones are captured at the start of the next block
+ * and written by a thread while it runs; the thread is joined before the next capture, so checkpoints are never
+ * skipped and a slow disk holds the run up. WDPM_B200_RESUME=<path> continues the run the file was written by, bit
+ * for bit: water, outlet totals, iteration count, drained total and initial volume come from it, the add or
+ * subtract step is skipped. A file that is missing, damaged or written by a run of another identity prints a
+ * message and exits with 1 before any solver exists.
  */
 #define _POSIX_C_SOURCE 200809L
 #include <ctype.h>
+#include <errno.h>
+#include <fcntl.h>
 #include <math.h>
 #include <pthread.h>
+#include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 #include <sys/stat.h>
 #include <sys/time.h>
+#include <unistd.h>
 
 #ifdef _OPENMP
 #include <omp.h>
@@ -489,7 +502,7 @@ static void die_solver(const char *what)
 
 /* ---- one solver, or one stripe solver per GPU ------------------------------- */
 
-enum { MAX_GPUS = 16, ENQUEUE_CHUNK = 50 };
+enum { MAX_GPUS = 16, ENQUEUE_CHUNK = 50, CK_HANDOVER_ITERATIONS = 200 };
 
 typedef struct {
     int n;                       /* solvers (1 = plain solver, >1 = row stripes) */
@@ -553,19 +566,37 @@ static void set_download(solver_set *ss, double *water, int cols)
         if (wdpm_download_water(ss->sv[g], water + (size_t)ss->owned_row0[g] * (size_t)cols) != WDPM_OK) die_solver("read water");
 }
 
-/* one block of `iters` iterations on every stripe; results combined in stripe order */
-static void set_run_block(solver_set *ss, int iters, wdpm_block_result *out)
+typedef struct ck_writer ck_writer;
+static void ck_hand_over(solver_set *ss, ck_writer *cw);
+
+/* One block of `iters` iterations on every stripe; results combined in stripe order. With `cw`, the solvers are
+ * armed: their capture lands while the first CK_HANDOVER_ITERATIONS run, and the host waits for it and hands it to
+ * the writer before feeding the rest. That many queued iterations keep every GPU busy during the wait (at 32768²
+ * on one GPU they take 1.4 s, the capture of 8.6 GB lands in 0.17 s), and the writer still has most of the
+ * block to write the file before the next capture is due. */
+static void set_run_block(solver_set *ss, int iters, wdpm_block_result *out, ck_writer *cw)
 {
-    if (ss->n == 1) {
+    if (ss->n == 1 && !cw) {
         if (wdpm_run_block(ss->sv[0], iters, out) != WDPM_OK) die_solver("run block");
         return;
     }
     for (int g = 0; g < ss->n; g++)
         if (wdpm_block_begin(ss->sv[g]) != WDPM_OK) die_solver("begin block");
-    for (int done = 0; done < iters; done += ENQUEUE_CHUNK) { /* feed all GPUs round-robin: nothing here blocks */
-        const int nit = iters - done < ENQUEUE_CHUNK ? iters - done : ENQUEUE_CHUNK;
+    int handed = !cw;
+    for (int done = 0; done < iters;) { /* feed all GPUs round-robin: nothing here blocks */
+        int nit = ss->n > 1 ? ENQUEUE_CHUNK : handed ? iters - done : CK_HANDOVER_ITERATIONS;
+        if (nit > iters - done) nit = iters - done;
         for (int g = 0; g < ss->n; g++)
             if (wdpm_block_enqueue(ss->sv[g], nit) != WDPM_OK) die_solver("enqueue iterations");
+        done += nit;
+        if (!handed && (done >= CK_HANDOVER_ITERATIONS || done == iters)) {
+            ck_hand_over(ss, cw);
+            handed = 1;
+        }
+    }
+    if (ss->n == 1) {
+        if (wdpm_block_end(ss->sv[0], out) != WDPM_OK) die_solver("end block");
+        return;
     }
     memset(out, 0, sizeof *out);
     for (int g = 0; g < ss->n; g++) {
@@ -625,6 +656,229 @@ static void mark_nodata(double *w, const double *dem, size_t n, double nodata)
         if (dem[k] <= nodata) w[k] = nodata;
 }
 
+/* ---- exact checkpoints (WDPM_B200_CHECKPOINT, WDPM_B200_RESUME) -----------------------------------------------
+ * The only code that knows the file format. Little-endian, in this order:
+ *   ck_header (128 bytes): magic, version, the run's identity, then where the run stands;
+ *   n_totals doubles: every outlet's drained total (depth in m, as the solver keeps it) in outlet order;
+ *   rows*cols doubles: the water, raw fp64 bits, row-major: the state the next block starts from;
+ *   a uint64 trailer: the water's order-free checksum (wdpm_water_checksum's definition).
+ * A checkpoint resumes only a run of the same identity: the DEM (size, nodata, georeference and a hash of its
+ * values' bits), module, schedule ("cpu" flag), depth, runoff fraction, zero threshold and outlet set. The elevation
+ * and drain tolerances, the iteration limit, paths, the GPU count and the kernel are free to change. */
+#define CK_MAGIC "WDPMCKPT"
+enum { CK_VERSION = 1 };
+
+typedef struct {
+    char magic[8];
+    uint32_t version;
+    int32_t module;                   /* WDPM_ADD / WDPM_SUBTRACT / WDPM_DRAIN */
+    int32_t rows, cols;
+    double nodata, cellsize, xll, yll;
+    uint64_t dem_hash;                /* ck_checksum of the DEM's fp64 bits */
+    int32_t schedule;                 /* WDPM_SCHEDULE_*, from the "cpu" flag */
+    int32_t n_totals;                 /* Drain: outlets (1 for the reference's outlet); 0 otherwise */
+    double depth, runoff_frac, thres; /* m, fraction, m */
+    uint64_t outlet_hash;             /* 0: the reference's outlet, or not Drain */
+    int64_t iterations;
+    double initial_vol, total_drain;  /* m3; m (the report's old_drain of the next block) */
+} ck_header;
+_Static_assert(sizeof(ck_header) == 128, "checkpoint header layout");
+
+/* sum of bits(g[k]) * (2 * (index0 + k) + 1) mod 2^64: equal sums over any partition of the same grid */
+static uint64_t ck_checksum(const double *g, size_t n, size_t index0)
+{
+    uint64_t sum = 0;
+#pragma omp parallel for reduction(+ : sum) schedule(static)
+    for (long long k = 0; k < (long long)n; k++) {
+        uint64_t b;
+        memcpy(&b, &g[k], sizeof b);
+        sum += b * (2 * ((uint64_t)index0 + (uint64_t)k) + 1);
+    }
+    return sum;
+}
+
+static uint64_t ck_outlet_hash(const outlet_set *os)
+{
+    if (os->n == 0) return 0;
+    uint64_t h = 1469598103934665603ull; /* FNV-1a over the (row, col) pairs in outlet order */
+    for (int32_t k = 0; k < os->n; k++) {
+        const int32_t v[2] = {os->row[k], os->col[k]};
+        const unsigned char *p = (const unsigned char *)v;
+        for (size_t b = 0; b < sizeof v; b++) h = (h ^ p[b]) * 1099511628211ull;
+    }
+    return h ? h : 1;
+}
+
+static void ck_identity(ck_header *h, const asc_header *hdr, const double *dem, int module, int schedule, double depth,
+                        double runoff_frac, double thres, const outlet_set *os)
+{
+    memset(h, 0, sizeof *h);
+    memcpy(h->magic, CK_MAGIC, sizeof h->magic);
+    h->version = CK_VERSION;
+    h->module = module;
+    h->rows = hdr->nrows;
+    h->cols = hdr->ncols;
+    h->nodata = hdr->nodata;
+    h->cellsize = hdr->cellsize;
+    h->xll = hdr->value[2];
+    h->yll = hdr->value[3];
+    h->dem_hash = ck_checksum(dem, (size_t)hdr->nrows * (size_t)hdr->ncols, 0);
+    h->schedule = schedule;
+    h->n_totals = module == WDPM_DRAIN ? (os->n > 0 ? os->n : 1) : 0;
+    h->depth = depth;
+    h->runoff_frac = runoff_frac;
+    h->thres = thres;
+    h->outlet_hash = ck_outlet_hash(os);
+}
+
+/* `pattern` with its first "%d" replaced by the iteration count */
+static void ck_path(char *out, size_t cap, const char *pattern, long long k)
+{
+    const char *p = strstr(pattern, "%d");
+    if (p) snprintf(out, cap, "%.*s%lld%s", (int)(p - pattern), pattern, k, p + 2);
+    else snprintf(out, cap, "%s", pattern);
+}
+
+/* One checkpoint to write: the water arrives in pieces of whole rows (a stripe's owned rows each, straight from the
+ * solvers' capture staging, or one piece for the whole grid) and each goes to its offset in the file. */
+struct ck_writer {
+    pthread_t thread;
+    int running, failed; /* failed: the errno of a failed write */
+    char path[1024];
+    ck_header h;
+    double *totals; /* h.n_totals */
+    int n_pieces;
+    const double *piece[MAX_GPUS];
+    int32_t row0[MAX_GPUS], nrows[MAX_GPUS];
+};
+
+static int pwrite_all(int fd, const void *buf, size_t len, off_t off)
+{
+    const char *p = buf;
+    while (len > 0) {
+        const ssize_t w = pwrite(fd, p, len < ((size_t)1 << 30) ? len : ((size_t)1 << 30), off);
+        if (w <= 0) {
+            if (w == 0) errno = EIO; /* no progress: a full device reports ENOSPC on the next call, but do not spin */
+            return -1;
+        }
+        p += w;
+        len -= (size_t)w;
+        off += w;
+    }
+    return 0;
+}
+
+/* A temporary file, fsync, then rename: the file at the path is always a complete checkpoint. Returns 0, or the
+ * errno of the first call that failed. */
+static int ck_write(ck_writer *cw)
+{
+    const ck_header *h = &cw->h;
+    char tmp[1100];
+    snprintf(tmp, sizeof tmp, "%s.tmp", cw->path);
+    const int fd = open(tmp, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (fd < 0) return errno ? errno : EIO;
+    const off_t water_at = (off_t)sizeof *h + (off_t)h->n_totals * (off_t)sizeof(double);
+    uint64_t sum = 0;
+    int err = 0;
+#define CK_CALL(ok) do { if (!err && !(ok)) err = errno ? errno : EIO; } while (0) /* later calls skipped once one fails */
+    CK_CALL(pwrite_all(fd, h, sizeof *h, 0) == 0);
+    CK_CALL(pwrite_all(fd, cw->totals, (size_t)h->n_totals * sizeof(double), (off_t)sizeof *h) == 0);
+    for (int p = 0; p < cw->n_pieces && !err; p++) {
+        const size_t cells = (size_t)cw->nrows[p] * (size_t)h->cols, first = (size_t)cw->row0[p] * (size_t)h->cols;
+        CK_CALL(pwrite_all(fd, cw->piece[p], cells * sizeof(double), water_at + (off_t)(first * sizeof(double))) == 0);
+        sum += ck_checksum(cw->piece[p], cells, first);
+    }
+    CK_CALL(pwrite_all(fd, &sum, sizeof sum, water_at + (off_t)((size_t)h->rows * (size_t)h->cols * sizeof(double))) == 0);
+    CK_CALL(fsync(fd) == 0);
+    if (close(fd) != 0 && !err) err = errno ? errno : EIO;
+    CK_CALL(rename(tmp, cw->path) == 0);
+#undef CK_CALL
+    if (err) unlink(tmp);
+    return err;
+}
+
+static void *ck_main(void *arg)
+{
+    ck_writer *cw = arg;
+    cw->failed = ck_write(cw);
+    return NULL;
+}
+
+/* Checkpoints are never skipped: a writer still busy when the next one is due holds the run up. */
+static void ck_join(ck_writer *cw)
+{
+    if (cw->running) {
+        pthread_join(cw->thread, NULL);
+        cw->running = 0;
+    }
+    if (cw->failed) {
+        fprintf(stderr, "Couldn't write the checkpoint %s: %s\n", cw->path, strerror(cw->failed));
+        exit(1);
+    }
+}
+
+static void ck_start(ck_writer *cw)
+{
+    if (pthread_create(&cw->thread, NULL, ck_main, cw) == 0) cw->running = 1;
+    else ck_main(cw);
+}
+
+/* Every solver's capture has landed: the writer takes their staging as it is (each stripe's rows go to their offset)
+ * and the totals added over the stripes (each lives on the stripe that owns its outlet and reads 0 on the others). */
+static void ck_hand_over(solver_set *ss, ck_writer *cw)
+{
+    for (int32_t q = 0; q < cw->h.n_totals; q++) cw->totals[q] = 0.0;
+    for (int g = 0; g < ss->n; g++) {
+        const void *w;
+        const double *t;
+        int32_t nt;
+        if (wdpm_checkpoint_wait(ss->sv[g], &w, &t, &nt) != WDPM_OK) die_solver("wait for the checkpoint capture");
+        cw->piece[g] = w;
+        cw->row0[g] = ss->owned_row0[g];
+        cw->nrows[g] = ss->owned_rows[g];
+        for (int32_t q = 0; q < cw->h.n_totals && q < nt; q++) cw->totals[q] += t[q];
+    }
+    cw->n_pieces = ss->n;
+    ck_start(cw);
+}
+
+static void ck_fail(const char *path, const char *why)
+{
+    fprintf(stderr, "Couldn't resume from the checkpoint WDPM_B200_RESUME=%s: %s\n", path, why);
+    exit(1);
+}
+
+/* Read the checkpoint at `path` into h, *totals (allocated) and water (rows*cols), refusing any file that is not a
+ * complete, intact checkpoint of a run with the identity `want`. */
+static void ck_read(const char *path, const ck_header *want, ck_header *h, double **totals, double *water)
+{
+    FILE *f = fopen(path, "rb");
+    if (!f) ck_fail(path, strerror(errno));
+    if (fread(h, sizeof *h, 1, f) != 1) ck_fail(path, "truncated file");
+    if (memcmp(h->magic, CK_MAGIC, sizeof h->magic) != 0) ck_fail(path, "not a checkpoint file (wrong magic)");
+    if (h->version != CK_VERSION) ck_fail(path, "unsupported checkpoint version");
+#define CK_SAME(field) (memcmp(&h->field, &want->field, sizeof h->field) == 0)
+    if (!CK_SAME(rows) || !CK_SAME(cols) || !CK_SAME(nodata) || !CK_SAME(cellsize) || !CK_SAME(xll) || !CK_SAME(yll) || !CK_SAME(dem_hash))
+        ck_fail(path, "it was written for another DEM");
+    if (!CK_SAME(module)) ck_fail(path, "it was written by another module");
+    if (!CK_SAME(schedule)) ck_fail(path, "it was written with another cpu flag (update schedule)");
+    if (!CK_SAME(depth) || !CK_SAME(runoff_frac)) ck_fail(path, "it was written with another depth or runoff fraction");
+    if (!CK_SAME(thres)) ck_fail(path, "it was written with another zero depth threshold");
+    if (!CK_SAME(n_totals) || !CK_SAME(outlet_hash)) ck_fail(path, "it was written with other drain outlets (WDPM_B200_OUTLETS)");
+#undef CK_SAME
+    if (h->iterations < 0 || h->iterations > INT32_MAX - 2 * BLOCK_ITERATIONS) ck_fail(path, "iteration count out of range");
+    const size_t n = (size_t)h->rows * (size_t)h->cols;
+    *totals = malloc(((size_t)h->n_totals + 1) * sizeof **totals);
+    if (!*totals) ck_fail(path, "out of memory");
+    uint64_t sum = 0;
+    if (fread(*totals, sizeof **totals, (size_t)h->n_totals, f) != (size_t)h->n_totals || fread(water, sizeof *water, n, f) != n ||
+        fread(&sum, sizeof sum, 1, f) != 1)
+        ck_fail(path, "truncated file");
+    if (fgetc(f) != EOF) ck_fail(path, "longer than a checkpoint");
+    fclose(f);
+    if (ck_checksum(water, n, 0) != sum) ck_fail(path, "checksum mismatch (the water grid is damaged)");
+}
+
 /* What a chained run carries from one module to the next (all of it owned here). */
 typedef struct {
     int active;
@@ -675,6 +929,11 @@ int main(int argc, char **argv)
     }
     if (argc >= 3 && !strcmp(argv[1], "chain")) { /* extension: several parameter files, one process */
         static chain_state cs;
+        for (const char *const *v = (const char *const[]){"WDPM_B200_CHECKPOINT", "WDPM_B200_RESUME", NULL}; *v; v++)
+            if (getenv(*v) && *getenv(*v)) {
+                fprintf(stderr, "%s does not apply to chain: checkpoint and resume one module at a time\n", *v);
+                return 1;
+            }
         cs.active = 1;
         for (int f = 2; f < argc; f++) {
             ntok = tokens_from_file(argv[f], tok, 16);
@@ -725,6 +984,18 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     const double eltol = a.eltol_mm / 1000.0;
     const double depth = is_add ? a.depth_mm / 1000.0 : a.depth_mm / 1000;
     const double thres = a.thres_mm / 1000;
+    /* exact checkpoints: written every ck_every blocks and at the end (ck_spec), or a run resumed from one */
+    const char *ck_spec = getenv("WDPM_B200_CHECKPOINT"), *resume_path = getenv("WDPM_B200_RESUME");
+    if (ck_spec && !*ck_spec) ck_spec = NULL;
+    if (resume_path && !*resume_path) resume_path = NULL;
+    int ck_every = 1;
+    if (getenv("WDPM_B200_CHECKPOINT_EVERY") && *getenv("WDPM_B200_CHECKPOINT_EVERY")) {
+        ck_every = atoi(getenv("WDPM_B200_CHECKPOINT_EVERY"));
+        if (ck_every < 1) {
+            fprintf(stderr, "WDPM_B200_CHECKPOINT_EVERY must be a positive number of blocks\n");
+            return 1;
+        }
+    }
 
     /* DEM header and data (a chained run keeps the DEM it parsed for the module before) */
     const int same_dem = cs && cs->dem && !strcmp(cs->dem_path, a.dem);
@@ -775,7 +1046,7 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     double *water = NULL;
     int resumed = 0, chained = 0; /* chained: the water file is the output the module before has just written */
     double initial_vol = 0.0;
-    if (!is_null_name(a.scratch)) {
+    if (!resume_path && !is_null_name(a.scratch)) {
         if (file_exists(a.scratch)) {
             line("           ");
             printf("%30s\n", "Scratch file found");
@@ -791,7 +1062,9 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
             line("           ");
         }
     }
-    if (!water) {
+    if (resume_path) {
+        water = malloc(n * sizeof *water); /* filled from the checkpoint once the outlets are known */
+    } else if (!water) {
         const int named = is_drain || !is_null_name(a.water);
         if (named && file_exists(a.water)) {
             printf("%30s\n", "Existing water file found");
@@ -819,7 +1092,7 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         perror("Couldn't read the water file");
         return 1;
     }
-    if (is_drain) {
+    if (is_drain && !resume_path) {
         initial_vol = 0.0;
         for (size_t k = 0; k < n; k++)
             if (dem[k] > nodata) initial_vol += water[k];
@@ -836,6 +1109,20 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     double *outlet_totals = os.n > 0 ? malloc((size_t)os.n * sizeof *outlet_totals) : NULL;
     if (os.n > 0 && !outlet_totals) outlets_fail(outlet_spec, "out of memory");
 
+    const int module = is_add ? WDPM_ADD : is_sub ? WDPM_SUBTRACT : WDPM_DRAIN;
+    const int schedule = a.backend == 0 ? WDPM_SCHEDULE_SERIAL : WDPM_SCHEDULE_OPENCL;
+    ck_header ident, ck_in;
+    double *ck_totals = NULL;
+    if (ck_spec || resume_path) ck_identity(&ident, &hdr, dem, module, schedule, is_drain ? 0.0 : depth, is_add ? a.runoff_frac : 0.0, thres, &os);
+    if (resume_path) { /* checked in full before any solver exists */
+        ck_read(resume_path, &ident, &ck_in, &ck_totals, water);
+        initial_vol = ck_in.initial_vol;
+        line("           ");
+        printf("%30s\n", "Checkpoint found");
+        printf("%30s %lld\n", "Resuming at iteration:", (long long)ck_in.iterations);
+        line("           ");
+    }
+
     /* solver */
     wdpm_config cfg;
     memset(&cfg, 0, sizeof cfg);
@@ -844,9 +1131,9 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     cfg.cols = cols;
     cfg.nodata = nodata;
     cfg.dtype = WDPM_F64;
-    cfg.module = is_add ? WDPM_ADD : is_sub ? WDPM_SUBTRACT : WDPM_DRAIN;
+    cfg.module = module;
     cfg.zero_threshold = thres;
-    cfg.schedule = a.backend == 0 ? WDPM_SCHEDULE_SERIAL : WDPM_SCHEDULE_OPENCL;
+    cfg.schedule = schedule;
     cfg.device = getenv("WDPM_B200_DEVICE") ? atoi(getenv("WDPM_B200_DEVICE")) : 0;
     cfg.kernel = getenv("WDPM_B200_KERNEL") ? atoi(getenv("WDPM_B200_KERNEL")) : WDPM_KERNEL_AUTO;
     solver_set ss;
@@ -866,7 +1153,7 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         for (int g = 0; g < cs->prev.n; g++) wdpm_destroy(cs->prev.sv[g]);
         cs->have_prev = 0;
     }
-    if (!resumed) {
+    if (!resumed && !resume_path) {
         for (int g = 0; g < ss.n; g++) {
             if (is_add && wdpm_apply_add(ss.sv[g], depth, a.runoff_frac) != WDPM_OK) die_solver("add water");
             if (is_sub && wdpm_apply_subtract(ss.sv[g], depth) != WDPM_OK) die_solver("subtract water");
@@ -882,9 +1169,10 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         }
         for (int g = 0; g < ss.n; g++) {
             if (wdpm_set_outlets(ss.sv[g], os.n, os.row, os.col) != WDPM_OK) die_solver("set the drain outlets");
-            if (wdpm_seed_outlet_drains(ss.sv[g]) != WDPM_OK) die_solver("seed the outlet totals");
+            if (resume_path ? wdpm_set_outlet_drains(ss.sv[g], ck_totals, os.n) != WDPM_OK : wdpm_seed_outlet_drains(ss.sv[g]) != WDPM_OK)
+                die_solver("seed the outlet totals");
         }
-        total_drain = set_outlet_totals(&ss, &os, outlet_totals);
+        total_drain = resume_path ? ck_in.total_drain : set_outlet_totals(&ss, &os, outlet_totals);
         line("               ");
         printf("%30s\n", "Basin summary");
         printf("%20s %10.4f %s\n", "Basin area:", (double)basincount * cellarea, "m2");
@@ -904,10 +1192,16 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         if (owner < 0) die_solver("locate the drain");
         for (int g = 0; g < ss.n; g++)
             if (wdpm_set_outlet(ss.sv[g], drow, dcol) != WDPM_OK) die_solver("set the drain");
-        if (wdpm_get_cell_water(ss.sv[owner], drow, dcol, &w_out) != WDPM_OK) die_solver("read the drain cell");
-        total_drain = w_out > 0 ? w_out : 0; /* WDPMCL.c:1029 */
-        for (int g = 0; g < ss.n; g++)
-            if (wdpm_set_total_drain(ss.sv[g], g == owner ? total_drain : 0.0) != WDPM_OK) die_solver("set totaldrain");
+        if (resume_path) {
+            total_drain = ck_in.total_drain;
+            for (int g = 0; g < ss.n; g++)
+                if (wdpm_set_outlet_drains(ss.sv[g], ck_totals, 1) != WDPM_OK) die_solver("set totaldrain");
+        } else {
+            if (wdpm_get_cell_water(ss.sv[owner], drow, dcol, &w_out) != WDPM_OK) die_solver("read the drain cell");
+            total_drain = w_out > 0 ? w_out : 0; /* WDPMCL.c:1029 */
+            for (int g = 0; g < ss.n; g++)
+                if (wdpm_set_total_drain(ss.sv[g], g == owner ? total_drain : 0.0) != WDPM_OK) die_solver("set totaldrain");
+        }
         line("               ");
         printf("%30s\n", "Basin summary");
         printf("%20s %10.4f %s\n", "Basin area:", (double)basincount * cellarea, "m2");
@@ -929,13 +1223,20 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
     /* blocks of 1000 iterations until a stop test fires (WDPMCL.c:1054-1377) */
     struct timeval t0;
     gettimeofday(&t0, NULL);
-    int k = 0, done = 0;
+    int k = resume_path ? (int)ck_in.iterations : 0, done = 0, armed = 0;
     scratch_writer scratch;
     memset(&scratch, 0, sizeof scratch);
+    static ck_writer ckw; /* large (per-GPU arrays); one module at a time */
+    memset(&ckw, 0, sizeof ckw);
+    if (ck_spec) {
+        ckw.totals = malloc(((size_t)ident.n_totals + 1) * sizeof *ckw.totals);
+        if (!ckw.totals) die_solver("allocate the checkpoint totals");
+    }
     while (!done) {
         const double old_drain = total_drain;
         wdpm_block_result r;
-        set_run_block(&ss, BLOCK_ITERATIONS, &r);
+        set_run_block(&ss, BLOCK_ITERATIONS, &r, armed ? &ckw : NULL);
+        armed = 0;
         k += BLOCK_ITERATIONS;
         total_drain = (os.n > 0 && ss.n > 1) ? set_outlet_totals(&ss, &os, outlet_totals) : r.total_drain;
         double diffdrain = 0.0;
@@ -952,12 +1253,40 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
             if (is_add) mark_nodata(water, dem, n, nodata);
             scratch_start(&scratch, a.scratch, &hdr, water, n);
         }
+        if (!done && ck_spec && (k / BLOCK_ITERATIONS) % ck_every == 0) { /* the next block captures the state at k */
+            ck_join(&ckw); /* its staging is about to be reused */
+            for (int g = 0; g < ss.n; g++)
+                if (wdpm_checkpoint_arm(ss.sv[g]) != WDPM_OK) die_solver("arm the checkpoint capture");
+            ckw.h = ident;
+            ckw.h.iterations = k;
+            ckw.h.initial_vol = initial_vol;
+            ckw.h.total_drain = total_drain;
+            ck_path(ckw.path, sizeof ckw.path, ck_spec, k);
+            armed = 1;
+        }
     }
 
     scratch_join(&scratch);
 
     /* final grid and statistics (WDPMCL.c:1379-1467) */
     set_download(&ss, water, cols);
+    if (ck_spec) { /* the end of the run, from the grid downloaded for the output anyway */
+        ck_join(&ckw);
+        ckw.h = ident;
+        ckw.h.iterations = k;
+        ckw.h.initial_vol = initial_vol;
+        ckw.h.total_drain = total_drain;
+        if (os.n > 0) set_outlet_totals(&ss, &os, ckw.totals);
+        else if (is_drain) ckw.totals[0] = total_drain;
+        ckw.n_pieces = 1;
+        ckw.piece[0] = water;
+        ckw.row0[0] = 0;
+        ckw.nrows[0] = rows;
+        ck_path(ckw.path, sizeof ckw.path, ck_spec, k);
+        ck_main(&ckw);
+        ck_join(&ckw);
+        free(ckw.totals);
+    }
     mark_nodata(water, dem, n, nodata);
     /* The order-free statistics come from the device (wdpm_final_statistics: counts add and maxima combine over the
      * stripes); the volume is the reference's own sequential sum over the grid the output file needs anyway, so that
@@ -1029,6 +1358,7 @@ static int run_module(int ntok, char tok[][512], int argc, chain_state *cs)
         }
     }
     free(outlet_totals);
+    free(ck_totals);
     free(os.row);
     free(os.col);
     free(scratch.grid);

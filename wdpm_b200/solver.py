@@ -128,6 +128,7 @@ class Solver:
         self.rows, self.cols, self.dtype, self.module, self.nodata = rows, cols, dtype, module, nodata
         self.schedule = schedule
         self.np_dtype = _np_dtype(dtype)
+        self.owned_rows = self.stripe.owned_rows if _stripe else rows  # interior rows download_water returns
 
     # -- lifetime ---------------------------------------------------------
     def close(self):
@@ -210,6 +211,26 @@ class Solver:
         out = np.zeros(n, dtype=np.float64)
         _check(self._lib.wdpm_get_outlet_drains(self._h, out.ctypes.data_as(C.POINTER(C.c_double)), C.c_int32(n)))
         return out
+
+    def set_outlet_drains(self, values):
+        """Restore every outlet's total, in the caller's order (on row stripes only the stripe that owns the outlet's
+        row keeps it)."""
+        v = np.ascontiguousarray(values, dtype=np.float64)
+        _check(self._lib.wdpm_set_outlet_drains(self._h, v.ctypes.data_as(C.POINTER(C.c_double)), C.c_int32(v.size)))
+
+    def checkpoint_arm(self):
+        """Capture the state the next block starts from (wdpm_checkpoint_arm)."""
+        _check(self._lib.wdpm_checkpoint_arm(self._h))
+
+    def checkpoint_wait(self):
+        """(water, totals) of the last capture, as copies: the owned interior rows in the solver's precision and the
+        outlet totals in the caller's order."""
+        w, t, n = C.c_void_p(), C.POINTER(C.c_double)(), C.c_int32()
+        _check(self._lib.wdpm_checkpoint_wait(self._h, C.byref(w), C.byref(t), C.byref(n)))
+        cells = self.owned_rows * self.cols
+        raw = (C.c_char * (cells * np.dtype(self.np_dtype).itemsize)).from_address(w.value)
+        water = np.frombuffer(raw, dtype=self.np_dtype).reshape(self.owned_rows, self.cols).copy()
+        return water, np.ctypeslib.as_array(t, shape=(n.value,)).copy()
 
     def quantize_water(self):
         """What a "%f" file hand-over does to the water grid (module chaining; include/wdpm_quantize.h)."""

@@ -158,6 +158,17 @@ class DistributedSolver:
     def seed_outlet_drains(self):
         self.solver.seed_outlet_drains()
 
+    def set_outlet_drains(self, values):
+        """Every stripe takes the whole array; the one that owns an outlet's row keeps its total."""
+        self.solver.set_outlet_drains(values)
+
+    def checkpoint_arm(self):
+        self.solver.checkpoint_arm()
+
+    def checkpoint_wait(self):
+        """This rank's capture: its owned rows and its share of the totals (0 for outlets of other stripes)."""
+        return self.solver.checkpoint_wait()
+
     def outlet_drains(self, n: int) -> np.ndarray:
         """Per-outlet totals of the whole DEM: each is kept by the stripe that owns the outlet's row (0 elsewhere),
         so the element-wise sum over the stripes is exact."""
