@@ -380,6 +380,22 @@ int fold_grid(const wdpm_solver* s) {
     return (int)std::min<long long>((n + 255) / 256, (long long)s->sm_count * 4);
 }
 
+// Row stripes: load, at creation, every kernel a stripe enqueues behind a k_halo_wait. With lazy module loading
+// (the CUDA default) a kernel's first launch loads it, and loading may wait for the kernels running on the device. On
+// one device, a stripe's k_halo_wait spins until its neighbour's iteration kernel has run; if the host is still in the
+// first launch of, say, k_fold_events for this stripe, it has not launched the neighbour's kernel yet, and the wait
+// ends only at its timeout (WDPM_E_HALO). cudaFuncGetAttributes loads the kernel without running it.
+template <typename T>
+cudaError_t preload_stripe_kernels() {
+    cudaFuncAttributes a;
+    cudaError_t e;
+    if ((e = cudaFuncGetAttributes(&a, (const void*)k_halo_wait)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&a, (const void*)k_block_prologue<T>)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&a, (const void*)k_gather_totals<T>)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&a, (const void*)k_outlet_wipe<T>)) != cudaSuccess) return e;
+    return cudaFuncGetAttributes(&a, (const void*)k_fold_events<T>);
+}
+
 int grid_for(long long n, int threads, int sm_count) {
     long long b = (n + threads - 1) / threads;
     const long long cap = (long long)sm_count * 16;
@@ -1045,6 +1061,10 @@ int wdpm_create(const wdpm_config* cfg, wdpm_solver** out) {
     }
 
     if (is_stripe && K != 1) { delete s; return fail(WDPM_E_UNSUPPORTED, "stripes need a fused variant with one iteration per launch"); }
+    if (is_stripe) {
+        e = s->dtype == WDPM_F64 ? preload_stripe_kernels<double>() : preload_stripe_kernels<float>();
+        if (e != cudaSuccess) { delete s; return fail(WDPM_E_CUDA, std::string("stripe kernel setup: ") + cudaGetErrorString(e)); }
+    }
     // the outlet's emptying sits between two iterations, and its event after the nine sub-pass slots of one iteration
     if (serial_drain(s) && s->kernel == WDPM_KERNEL_FUSED && K != 1) { delete s; return fail(WDPM_E_UNSUPPORTED, "serial-schedule Drain needs a fused variant with one iteration per launch"); }
 

@@ -516,7 +516,7 @@ static void set_create(solver_set *ss, wdpm_config base, int want)
     int n = want;
     if (n > MAX_GPUS) n = MAX_GPUS;
     if (n > wdpm_device_count() - base.device) n = wdpm_device_count() - base.device;
-    while (n > 1 && triples < 3 * n) n--; /* a stripe needs at least 9 rows */
+    while (n > 1 && padded < 9 * n) n--; /* a stripe needs at least 9 rows (3 * n triples are too few when the last is partial) */
     if (n < 1) n = 1;
     memset(ss, 0, sizeof *ss);
     ss->n = n;

@@ -29,10 +29,12 @@ class Stripe:
 
 
 def plan_stripes(rows: int, n: int) -> list[Stripe]:
-    """Cut padded rows 0..rows+1 into n contiguous bands starting at multiples of 3, as equal as possible."""
+    """Cut padded rows 0..rows+1 into n contiguous bands starting at multiples of 3, as equal as possible.
+    Every band gets at least 9 rows (HALO_ABOVE + HALO_BELOW), which needs 9 * n padded rows: 3 * n row triples are
+    not enough when the last one is partial, the last band would get 7 or 8 rows."""
     padded = rows + 2
     triples = (padded + 2) // 3
-    if n < 1 or triples < 3 * n:
+    if n < 1 or padded < 9 * n:
         raise ValueError(f"{rows} rows are too few for {n} stripes")
     out = []
     for r in range(n):
